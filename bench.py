@@ -1,13 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 leapfrog engine (contract: see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch: the fused L=32-step leapfrog trajectory
 (`step(Leapfrog(0.1), h, z, 32)`, src/integrator.jl:216-265) of 4096 chains x D=128 on a diagonal Gaussian
 target with a Diag-Euclidean metric -- the configuration BASELINE.json's metric is quoted on.
 Metric: leapfrog-steps*dims/s.  Weak scaling: every rank runs the same 4096-chain batch (chains shard
 with no data-path collective, SURVEY 8e), value = all ranks' units / max-over-ranks device time.
+
+--dump-outputs DIR writes the phase point the last timed step returned (rank 0; float64, 12.6 MB) as DIR/<name>.npy.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -64,6 +67,12 @@ def measured_traffic():
         return None
 
 
+def save_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.ascontiguousarray(v, dtype=np.float64))
+
+
 class Extra:
     """an extra measurement that fails is reported under "extras_failed" -- it must never cost the headline line"""
     errors = {}
@@ -107,6 +116,7 @@ class ClockSampler:
             return None
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()
         sm, reasons, mx = [], set(), None
         for r in self.rows:
             try:
@@ -201,6 +211,11 @@ def run_reference(args):
     for _ in range(args.steps):
         oc.leapfrog_omp(om, ome, EPS, z0, L_STEPS, n_threads=cores, out=out)
     dt = time.perf_counter() - t0
+    # the oracle's (D, N) column-major arrays, stored in the (N, D) layout of the GPU arm; this arm's model has no
+    # normalising constant, so its lp_value differs from the GPU arm's by -D/2 log(2 pi) - sum(log s)
+    if args.dump_outputs:
+        save_outputs(args.dump_outputs, {"theta": out.theta.T, "r": out.r.T, "lp_value": out.lp_value,
+                                         "lp_gradient": out.lp_gradient.T, "lk_value": out.lk_value})
     value = units * args.steps / dt
     extra = cpu_baselines(m, s, Minv, th, r, full=True)
     line = {
@@ -265,21 +280,29 @@ def run_ours(args):
         torch.cuda.synchronize()
         sampler = ClockSampler(local)
         sampler.start()
-        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
-        l0 = ctx.launches
-        for i in range(K):
-            flush_l2()  # L2 flush between timed iterations (outside the event pair)
-            ev[i][0].record(stream)
-            one_step()
-            ev[i][1].record(stream)
-        torch.cuda.synchronize()
-        launches = ctx.launches - l0
-        # keep the sampler alive for a moment of sustained load so clocks are seen under load
-        t_end = time.time() + 0.4
-        while time.time() < t_end:
-            one_step()
-        torch.cuda.synchronize()
-        clocks = sampler.stop()
+        try:
+            ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
+            l0 = ctx.launches
+            for i in range(K):
+                flush_l2()  # L2 flush between timed iterations (outside the event pair)
+                ev[i][0].record(stream)
+                zt = one_step()
+                ev[i][1].record(stream)
+            dumped = None
+            if args.dump_outputs and rank == 0:  # copied on the stream before the untimed steps below overwrite them
+                dumped = {"theta": zt.theta.clone(), "r": zt.r.clone(), "lp_value": zt.lp.value.clone(),
+                          "lp_gradient": zt.lp.gradient.clone(), "lk_value": zt.lk.value.clone()}
+            torch.cuda.synchronize()
+            launches = ctx.launches - l0
+            # keep the sampler alive for a moment of sustained load so clocks are seen under load
+            t_end = time.time() + 0.4
+            while time.time() < t_end:
+                one_step()
+            torch.cuda.synchronize()
+        finally:
+            clocks = sampler.stop()
+        if dumped is not None:
+            save_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in dumped.items()})
         if world > 1:
             dist.barrier()
         step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -735,7 +758,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     with StdoutToStderr() as out:
         args.emit = out.emit
         if args.impl == "reference":
