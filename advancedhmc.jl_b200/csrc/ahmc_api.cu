@@ -23,6 +23,11 @@
 
 using namespace ahmc;
 
+struct DevBuf {  // grow-only device buffer (see grow())
+    char* p = nullptr;
+    size_t bytes = 0;
+};
+
 struct ahmc_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -30,20 +35,13 @@ struct ahmc_ctx {
     std::string err;
     int64_t launches = 0;
     int* d_min_break = nullptr;   // device int for COMPAT_BREAK_ALL
-    char* arena = nullptr;        // grow-only device arena used by HOST_BUFFERS staging
-    size_t arena_bytes = 0;
-    double* nuts_scratch = nullptr;  // per-chain NUTS tree workspace
-    size_t nuts_scratch_bytes = 0;
-    double* adapt_scratch = nullptr;
-    size_t adapt_scratch_bytes = 0;
-    double* mn_scratch = nullptr;  // multinomial-static per-chain energy tape
-    size_t mn_scratch_bytes = 0;
-    char* dense_scratch = nullptr;  // K4: padded Minv, norms, per-chain fallback mask
-    double* coop_scratch = nullptr;  // cooperative NUTS products: Minv and cholU with padded columns (coop_lds)
-    size_t coop_scratch_doubles = 0;
-    size_t dense_scratch_bytes = 0;
-    char* split_scratch = nullptr;   // callback (split-step) mode workspace
-    size_t split_scratch_bytes = 0;
+    DevBuf arena;          // HOST_BUFFERS staging
+    DevBuf nuts_scratch;   // per-chain NUTS tree workspace
+    DevBuf adapt_scratch;  // adaptor statistics: last-block counter, per-block partials
+    DevBuf mn_scratch;     // multinomial-static per-chain energy tape
+    DevBuf dense_scratch;  // K4: padded Minv, norms, per-chain fallback mask
+    DevBuf coop_scratch;   // cooperative NUTS products: Minv and cholU with padded columns (coop_lds)
+    DevBuf split_scratch;  // callback (split-step) mode workspace
     // host-buffer pipeline: H2D stream, compute stream (= stream), D2H stream, one event pair per chunk
     static constexpr int kMaxPipeChunks = 32, kPipeStreams = 5;  // 3 upload, 1 download, 1 second compute
     cudaStream_t pipe[kPipeStreams] = {};
@@ -114,90 +112,83 @@ struct DeviceGuard {
     }
 };
 
-// Maps caller arrays to device arrays.  Device-pointer mode: identity.  HOST_BUFFERS mode: bump-allocates
-// from the context arena, copies inputs host->device on the context stream and outputs device->host in finish().
+constexpr size_t al256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// Grows `b` to at least `need` bytes (allocating `cap` >= need, default need).  Queued work may still use the old
+// allocation, so every stream of the context is drained before it is freed.
+int grow(ahmc_ctx* ctx, DevBuf& b, size_t need, const char* what, size_t cap = 0) {
+    if (need <= b.bytes) return AHMC_OK;
+    if (b.p) {
+        CU(cudaStreamSynchronize(ctx->stream));
+        for (cudaStream_t s : ctx->pipe)
+            if (s) CU(cudaStreamSynchronize(s));
+        CU(cudaFree(b.p));
+        b.p = nullptr;
+        b.bytes = 0;
+    }
+    if (cap < need) cap = need;
+    if (cudaMalloc((void**)&b.p, cap) != cudaSuccess) {
+        b.p = nullptr;
+        return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the %s failed", cap, what);
+    }
+    b.bytes = cap;
+    return AHMC_OK;
+}
+
+// Maps caller arrays to device arrays.  Device-pointer mode: identity, set at once (nothing is recorded, so that path
+// never allocates).  HOST_BUFFERS mode: in / out / inout record the array; commit() carves every recorded array from
+// the context arena, sets the device pointers and copies the inputs host->device on the context stream; finish()
+// copies the outputs device->host.  Staged device pointers exist only after commit().
 class Stager {
 public:
     Stager(ahmc_ctx* c, bool host) : ctx_(c), host_(host) {}
-    // first pass: reserve; second pass: bind.  (two passes so the arena is sized before any copy)
-    size_t need = 0;
-    // `bytes` may cover several arrays that are later carved one by one (each rounded up to 256 B on its own):
-    // kSlack pays for those roundings (every call site stages fewer than kSlack / 256 arrays)
-    static constexpr size_t kSlack = 64 * 256;
-    void reserve(size_t bytes) { need += (bytes + 255) & ~(size_t)255; }
-    int prepare() {
-        if (!host_) return AHMC_OK;
+    template <class T>
+    void in(const T* h, size_t count, const T** d) { add(h, count * sizeof(T), d, true, false); }
+    template <class T>
+    void out(T* h, size_t count, T** d) { add(h, count * sizeof(T), d, false, true); }
+    template <class T>
+    void inout(T* h, size_t count, T** d) { add(h, count * sizeof(T), d, true, true); }
+    int commit() {
+        if (reqs_.empty()) return AHMC_OK;
         ahmc_ctx* ctx = ctx_;
-        need += kSlack;
-        if (need > ctx->arena_bytes) {
-            if (ctx->arena) {
-                CU(cudaStreamSynchronize(ctx->stream));
-                CU(cudaFree(ctx->arena));
-                ctx->arena = nullptr;
-                ctx->arena_bytes = 0;
-            }
-            size_t cap = need + need / 4;
-            cudaError_t e = cudaMalloc((void**)&ctx->arena, cap);
-            if (e != cudaSuccess) return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for staging failed: %s", cap, cudaGetErrorString(e));
-            ctx->arena_bytes = cap;
+        size_t need = 0;
+        for (const Req& r : reqs_) need += al256(r.bytes);
+        int rc = grow(ctx, ctx->arena, need, "staging arena", need + need / 4);
+        if (rc) return rc;
+        char* p = ctx->arena.p;
+        for (Req& r : reqs_) {
+            r.dev = p;
+            set(r.slot, p);
+            if (r.in) CU(cudaMemcpyAsync(p, r.h, r.bytes, cudaMemcpyHostToDevice, ctx->stream));
+            p += al256(r.bytes);
         }
-        off_ = 0;
-        return AHMC_OK;
-    }
-    template <class T>
-    int in(const T* h, size_t count, const T** d) {
-        if (!h) { *d = nullptr; return AHMC_OK; }
-        if (!host_) { *d = h; return AHMC_OK; }
-        ahmc_ctx* ctx = ctx_;
-        T* p = (T*)alloc(count * sizeof(T));
-        if (!p) return overflow();
-        CU(cudaMemcpyAsync(p, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-        *d = p;
-        return AHMC_OK;
-    }
-    template <class T>
-    int out(T* h, size_t count, T** d) {
-        if (!h) { *d = nullptr; return AHMC_OK; }
-        if (!host_) { *d = h; return AHMC_OK; }
-        T* p = (T*)alloc(count * sizeof(T));
-        if (!p) return overflow();
-        outs_.push_back({(void*)h, (void*)p, count * sizeof(T)});
-        *d = p;
-        return AHMC_OK;
-    }
-    template <class T>
-    int inout(T* h, size_t count, T** d) {  // copied in now, copied back at finish
-        if (!h) { *d = nullptr; return AHMC_OK; }
-        if (!host_) { *d = h; return AHMC_OK; }
-        ahmc_ctx* ctx = ctx_;
-        T* p = (T*)alloc(count * sizeof(T));
-        if (!p) return overflow();
-        CU(cudaMemcpyAsync(p, h, count * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-        outs_.push_back({(void*)h, (void*)p, count * sizeof(T)});
-        *d = p;
         return AHMC_OK;
     }
     int finish() {
         ahmc_ctx* ctx = ctx_;
-        for (auto& o : outs_) CU(cudaMemcpyAsync(o.h, o.d, o.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        for (const Req& r : reqs_)
+            if (r.out) CU(cudaMemcpyAsync((void*)r.h, r.dev, r.bytes, cudaMemcpyDeviceToHost, ctx->stream));
         return AHMC_OK;
     }
     bool host() const { return host_; }
 
 private:
-    struct Out { void* h; void* d; size_t bytes; };
-    void* alloc(size_t bytes) {  // nullptr when the reservation pass undercounted: never hand out memory past the arena
-        const size_t b = (bytes + 255) & ~(size_t)255;
-        if (off_ + b > ctx_->arena_bytes) return nullptr;
-        void* p = ctx_->arena + off_;
-        off_ += b;
-        return p;
+    struct Req {
+        const void* h;
+        size_t bytes;
+        void* slot;  // the caller's T* that receives the device pointer
+        bool in, out;
+        void* dev;
+    };
+    // the slot is a T* of the caller's type: written bytewise, not through a void* lvalue
+    static void set(void* slot, const void* p) { memcpy(slot, &p, sizeof p); }
+    void add(const void* h, size_t bytes, void* slot, bool in, bool out) {
+        if (!h || !host_) set(slot, h);
+        else reqs_.push_back({h, bytes, slot, in, out, nullptr});
     }
-    int overflow() { return fail(ctx_, AHMC_ERR_NOMEM, "internal: host-buffer staging arena undersized (%zu of %zu bytes used)", off_, ctx_->arena_bytes); }
     ahmc_ctx* ctx_;
     bool host_;
-    size_t off_ = 0;
-    std::vector<Out> outs_;
+    std::vector<Req> reqs_;
 };
 
 int check_common(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* metric, int32_t D, int64_t N, bool streaming_ok = false) {
@@ -250,18 +241,13 @@ size_t metric_minv_count(const ahmc_metric* m, int32_t D, int64_t N) {
 ModelDev model_dev(const ahmc_model* m) { return ModelDev{m->kind, m->D, m->d_p0, m->d_p1, m->c0, m->rtc, m->d_p1_coop}; }
 
 // stage the metric descriptor (device or host pointers) into a MetricDev
-int stage_metric(Stager& st, const ahmc_metric* m, int32_t D, int64_t N, MetricDev* out) {
+void stage_metric(Stager& st, const ahmc_metric* m, int32_t D, int64_t N, MetricDev* out) {
     out->kind = m->kind;
     out->chain_stride = m->kind == AHMC_METRIC_DIAG ? m->chain_stride : 0;
     out->Minv_coop = nullptr;
     out->cholU_coop = nullptr;
-    int rc = st.in(m->Minv, metric_minv_count(m, D, N), &out->Minv);
-    if (rc) return rc;
-    return st.in(m->kind == AHMC_METRIC_DENSE ? m->cholU : (const double*)nullptr, (size_t)D * D, &out->cholU);
-}
-void reserve_metric(Stager& st, const ahmc_metric* m, int32_t D, int64_t N) {
-    st.reserve(metric_minv_count(m, D, N) * sizeof(double));
-    if (m->kind == AHMC_METRIC_DENSE) st.reserve((size_t)D * D * sizeof(double));
+    st.in(m->Minv, metric_minv_count(m, D, N), &out->Minv);
+    st.in(m->kind == AHMC_METRIC_DENSE ? m->cholU : (const double*)nullptr, (size_t)D * D, &out->cholU);
 }
 
 int finish_call(ahmc_ctx* ctx, Stager& st, uint32_t flags) {
@@ -284,25 +270,17 @@ struct SplitWork {
 };
 
 int split_workspace(ahmc_ctx* ctx, int32_t D, int64_t N, int64_t ld, SplitWork* w) {
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t need = al((size_t)N * 8) + al((size_t)ld * N * 8) + al((size_t)D * N * 8) + al((size_t)N * 8) +
-                        al((size_t)N * 4) * 2 + 256;
-    if (need > ctx->split_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->split_scratch);
-        ctx->split_scratch = nullptr;
-        ctx->split_scratch_bytes = 0;
-        if (cudaMalloc((void**)&ctx->split_scratch, need) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the split-step workspace failed", need);
-        ctx->split_scratch_bytes = need;
-    }
-    char* p = ctx->split_scratch;
-    w->cb_lp = (double*)p; p += al((size_t)N * 8);
-    w->cb_grad = (double*)p; p += al((size_t)ld * N * 8);
-    w->r0 = (double*)p; p += al((size_t)D * N * 8);
-    w->lk0 = (double*)p; p += al((size_t)N * 8);
-    w->status = (uint32_t*)p; p += al((size_t)N * 4);
-    w->steps = (int32_t*)p; p += al((size_t)N * 4);
+    const size_t need = al256((size_t)N * 8) + al256((size_t)ld * N * 8) + al256((size_t)D * N * 8) + al256((size_t)N * 8) +
+                        al256((size_t)N * 4) * 2 + 256;
+    int rc = grow(ctx, ctx->split_scratch, need, "split-step workspace");
+    if (rc) return rc;
+    char* p = ctx->split_scratch.p;
+    w->cb_lp = (double*)p; p += al256((size_t)N * 8);
+    w->cb_grad = (double*)p; p += al256((size_t)ld * N * 8);
+    w->r0 = (double*)p; p += al256((size_t)D * N * 8);
+    w->lk0 = (double*)p; p += al256((size_t)N * 8);
+    w->status = (uint32_t*)p; p += al256((size_t)N * 4);
+    w->steps = (int32_t*)p; p += al256((size_t)N * 4);
     w->flag = (int*)p;
     return AHMC_OK;
 }
@@ -353,35 +331,32 @@ int split_trajectory(ahmc_ctx* ctx, const ahmc_model* model, const MetricDev& md
     return AHMC_OK;
 }
 
-// K4 dispatch: GEMM-shaped operators (dense metric and/or dense-Gaussian target) -> tiled DMMA kernel; chains of tiles it
-// declines (magnitude proof not met) are redone by the exact warp-per-chain kernel from the untouched inputs.
-// `a` holds DEVICE pointers.  Returns 1 if handled, 0 if the configuration is not eligible, < 0 on error.
-int try_dense_trajectory(ahmc_ctx* ctx, const ahmc_model* model, LeapfrogArgs& a, int n_abs, double eps, double temper_alpha,
-                         bool compat, int* nl) {
-    const int D = a.D;
-    const long long N = a.N;
+// K4 (tiled DMMA trajectory) takes GEMM-shaped operators: a Gaussian target, a metric shared by all chains, a dense
+// matrix on either side, a tile shape for D, and neither exact checks, tempering nor COMPAT_BREAK_ALL.
+bool dense_eligible(const ahmc_model* model, const MetricDev& metric, uint32_t flags, double temper_alpha, bool compat,
+                    bool has_g, int32_t D) {
     const bool gauss = model->kind == AHMC_MODEL_STD_NORMAL || model->kind == AHMC_MODEL_DIAG_GAUSS ||
                        model->kind == AHMC_MODEL_DENSE_GAUSS;
-    const bool metric_ok = a.metric.kind != AHMC_METRIC_DIAG || a.metric.chain_stride == 0;
-    const bool has_dense = model->kind == AHMC_MODEL_DENSE_GAUSS || a.metric.kind == AHMC_METRIC_DENSE;
+    const bool metric_ok = metric.kind != AHMC_METRIC_DIAG || metric.chain_stride == 0;
+    const bool has_dense = model->kind == AHMC_MODEL_DENSE_GAUSS || metric.kind == AHMC_METRIC_DENSE;
     int Dp, RB, CB;
-    if (!(gauss && metric_ok && has_dense && !compat && a.g_in && !(a.flags & AHMC_FLAG_EXACT_CHECKS) && !(temper_alpha > 0.0) &&
-          dense_tile_shape(D, &Dp, &RB, &CB) && (model->kind != AHMC_MODEL_DENSE_GAUSS || model->d_p1_pad)))
-        return 0;
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t need = al(dense_mat_doubles(Dp) * 8) + al(16) + al((size_t)N);
-    if (need > ctx->dense_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->dense_scratch);
-        ctx->dense_scratch = nullptr;
-        ctx->dense_scratch_bytes = 0;
-        if (cudaMalloc((void**)&ctx->dense_scratch, need) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the dense workspace failed", need);
-        ctx->dense_scratch_bytes = need;
-    }
-    double* Mpad = (double*)ctx->dense_scratch;
-    double* norms = (double*)(ctx->dense_scratch + al(dense_mat_doubles(Dp) * 8));
-    uint8_t* mask = (uint8_t*)(ctx->dense_scratch + al(dense_mat_doubles(Dp) * 8) + al(16));
+    return gauss && metric_ok && has_dense && !compat && has_g && !(flags & AHMC_FLAG_EXACT_CHECKS) && !(temper_alpha > 0.0) &&
+           dense_tile_shape(D, &Dp, &RB, &CB) && (model->kind != AHMC_MODEL_DENSE_GAUSS || model->d_p1_pad);
+}
+
+// K4 trajectory of a dense_eligible configuration; chains of tiles it declines (magnitude proof not met) are redone by
+// the exact warp-per-chain kernel from the untouched inputs.  `a` holds DEVICE pointers.
+int dense_trajectory(ahmc_ctx* ctx, const ahmc_model* model, const LeapfrogArgs& a, int n_abs, double eps, int* nl) {
+    const int D = a.D;
+    const long long N = a.N;
+    int Dp, RB, CB;
+    dense_tile_shape(D, &Dp, &RB, &CB);
+    const size_t need = al256(dense_mat_doubles(Dp) * 8) + al256(16) + al256((size_t)N);
+    int rc = grow(ctx, ctx->dense_scratch, need, "dense workspace");
+    if (rc) return rc;
+    double* Mpad = (double*)ctx->dense_scratch.p;
+    double* norms = (double*)(ctx->dense_scratch.p + al256(dense_mat_doubles(Dp) * 8));
+    uint8_t* mask = (uint8_t*)(ctx->dense_scratch.p + al256(dense_mat_doubles(Dp) * 8) + al256(16));
     DenseTrajHost h{};
     h.D = D; h.Dp = Dp; h.N = N; h.c0 = model->c0;
     h.mu = (model->kind == AHMC_MODEL_STD_NORMAL) ? nullptr : model->d_p0;
@@ -413,7 +388,87 @@ int try_dense_trajectory(ahmc_ctx* ctx, const ahmc_model* model, LeapfrogArgs& a
     b.only_mask = mask;
     b.min_break = nullptr;
     CU(launch_leapfrog(b, ctx->stream, nl));
-    return 1;
+    return AHMC_OK;
+}
+
+// D x N column block copy between arrays of leading dimensions ldd / lds (nothing to do in place)
+int copy_cols(ahmc_ctx* ctx, double* dst, int64_t ldd, const double* src, int64_t lds, int32_t D, int64_t N,
+              cudaMemcpyKind kind = cudaMemcpyDeviceToDevice) {
+    if (!dst || !src || dst == src) return AHMC_OK;
+    CU(cudaMemcpy2DAsync(dst, (size_t)ldd * 8, src, (size_t)lds * 8, (size_t)D * 8, (size_t)N, kind, ctx->stream));
+    return AHMC_OK;
+}
+
+int check_rng_alphas(ahmc_ctx* ctx, const ahmc_rng* rng) {
+    if (!(rng->partial_refresh_alpha > -1.0 && rng->partial_refresh_alpha < 1.0))
+        return fail(ctx, AHMC_ERR_INVALID, "partial_refresh_alpha must be in (-1, 1)");
+    if (!(rng->temper_alpha >= 0.0) || std::isinf(rng->temper_alpha))
+        return fail(ctx, AHMC_ERR_INVALID, "temper_alpha must be 0 (plain Leapfrog) or a finite alpha > 0 (TemperedLeapfrog)");
+    return AHMC_OK;
+}
+
+int check_transition_output(ahmc_ctx* ctx, const ahmc_metric* metric, const ahmc_phasepoint* z_out, uint32_t flags) {
+    if (metric->kind == AHMC_METRIC_DENSE && !metric->cholU && !(flags & AHMC_FLAG_NO_REFRESH))
+        return fail(ctx, AHMC_ERR_INVALID, "Dense metric needs cholU for the momentum refresh (metric.jl:311-320)");
+    if (z_out->lk_gradient)
+        return fail(ctx, AHMC_ERR_UNSUPPORTED, "transition entry points do not emit lk_gradient; call ahmc_phasepoint_f64 if needed");
+    return AHMC_OK;
+}
+
+// a transition reads (theta, r, -grad lp, lp) of z_in and writes (theta, r, -grad lp, lp, lk) of z_out; `Args` is any
+// argument block with these fields (LeapfrogArgs, NutsArgs, MultinomialArgs)
+template <class Args>
+void stage_transition_pp(Stager& st, const ahmc_phasepoint* z_in, const ahmc_phasepoint* z_out, int64_t N, Args& a) {
+    const size_t cin = (size_t)z_in->ld * N, cout = (size_t)z_out->ld * N;
+    a.ld_in = z_in->ld;
+    a.ld_out = z_out->ld;
+    st.in((const double*)z_in->theta, cin, &a.th_in);
+    st.in((const double*)z_in->r, cin, &a.r_in);
+    st.in((const double*)z_in->lp_gradient, cin, &a.g_in);
+    st.in((const double*)z_in->lp_value, (size_t)N, &a.lp_in);
+    st.out(z_out->theta, cout, &a.th_out);
+    st.out(z_out->r, cout, &a.r_out);
+    st.out(z_out->lp_gradient, cout, &a.g_out);
+    st.out(z_out->lp_value, (size_t)N, &a.lp_out);
+    st.out(z_out->lk_value, (size_t)N, &a.lk_out);
+}
+
+void stage_stats(Stager& st, const ahmc_stats* s, int64_t N, StatsDev* d) {
+    memset(d, 0, sizeof *d);
+    if (!s) return;
+    st.out(s->n_steps, (size_t)N, &d->n_steps);
+    st.out(s->is_accept, (size_t)N, &d->is_accept);
+    st.out(s->acceptance_rate, (size_t)N, &d->acceptance_rate);
+    st.out(s->log_density, (size_t)N, &d->log_density);
+    st.out(s->hamiltonian_energy, (size_t)N, &d->hamiltonian_energy);
+    st.out(s->hamiltonian_energy_error, (size_t)N, &d->hamiltonian_energy_error);
+    st.out(s->max_hamiltonian_energy_error, (size_t)N, &d->max_hamiltonian_energy_error);
+    st.out(s->tree_depth, (size_t)N, &d->tree_depth);
+    st.out(s->numerical_error, (size_t)N, &d->numerical_error);
+}
+
+void stage_rng(Stager& st, const ahmc_rng* r, int32_t D, int64_t N, bool nuts, RngDev* d) {
+    d->seed = r->seed;
+    d->offset = r->offset;
+    d->partial_alpha = r->partial_refresh_alpha;
+    d->temper_alpha = r->temper_alpha > 0.0 ? r->temper_alpha : 0.0;
+    d->exp_stride = nuts ? r->exp_stride : 1;
+    d->dir_stride = r->dir_stride;
+    st.in(r->normal_tape, (size_t)D * N, &d->normal_tape);
+    st.in(r->exp_tape, (size_t)(nuts ? r->exp_stride : 1) * N, &d->exp_tape);
+    st.in(nuts ? r->dir_tape : (const uint8_t*)nullptr, (size_t)r->dir_stride * N, &d->dir_tape);
+}
+
+// adaptor-statistics workspace: [last-block counter (as 2 doubles)] [per-block partials].  Zeroed whenever it is
+// (re)allocated; after that the kernel re-arms the counter at the end of every launch.
+int adapt_workspace(ahmc_ctx* ctx, int32_t D, int64_t N, int* blocks) {
+    *blocks = (int)(N < 148 ? N : 148);
+    const size_t need = ((size_t)*blocks * (D + 1) + 2) * sizeof(double);
+    if (need <= ctx->adapt_scratch.bytes) return AHMC_OK;
+    int rc = grow(ctx, ctx->adapt_scratch, need, "adaptor workspace");
+    if (rc) return rc;
+    CU(cudaMemsetAsync(ctx->adapt_scratch.p, 0, need, ctx->stream));
+    return AHMC_OK;
 }
 }  // namespace
 
@@ -460,13 +515,9 @@ int ahmc_destroy(ahmc_ctx* ctx) {
     DeviceGuard g(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     cudaFree(ctx->d_min_break);
-    cudaFree(ctx->arena);
-    cudaFree(ctx->nuts_scratch);
-    cudaFree(ctx->adapt_scratch);
-    cudaFree(ctx->mn_scratch);
-    cudaFree(ctx->dense_scratch);
-    cudaFree(ctx->coop_scratch);
-    cudaFree(ctx->split_scratch);
+    for (DevBuf* b : {&ctx->arena, &ctx->nuts_scratch, &ctx->adapt_scratch, &ctx->mn_scratch, &ctx->dense_scratch,
+                      &ctx->coop_scratch, &ctx->split_scratch})
+        cudaFree(b->p);
     for (int i = 0; i < ahmc_ctx::kPipeStreams; ++i) {
         if (ctx->pipe[i]) cudaStreamDestroy(ctx->pipe[i]);
         if (ctx->ev_join[i]) cudaEventDestroy(ctx->ev_join[i]);
@@ -635,23 +686,19 @@ int ahmc_phasepoint_f64(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metri
     if (N == 0) return AHMC_OK;
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    const size_t DN = (size_t)z->ld * N * sizeof(double), Nb = (size_t)N * sizeof(double);
-    reserve_metric(st, metric, D, N);
-    st.reserve(DN * 4);
-    st.reserve(Nb * 2);
-    if ((rc = st.prepare())) return rc;
     PhasepointArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D;
     a.N = N;
     a.ld = z->ld;
-    if ((rc = st.in((const double*)z->theta, (size_t)z->ld * N, &a.th))) return rc;
-    if ((rc = st.in((const double*)z->r, (size_t)z->ld * N, &a.r))) return rc;
-    if ((rc = st.out(z->lp_value, (size_t)N, &a.lp))) return rc;
-    if ((rc = st.out(z->lp_gradient, (size_t)z->ld * N, &a.g))) return rc;
-    if ((rc = st.out(z->lk_value, (size_t)N, &a.lk))) return rc;
-    if ((rc = st.out(z->lk_gradient, (size_t)z->ld * N, &a.dr))) return rc;
+    st.in((const double*)z->theta, (size_t)z->ld * N, &a.th);
+    st.in((const double*)z->r, (size_t)z->ld * N, &a.r);
+    st.out(z->lp_value, (size_t)N, &a.lp);
+    st.out(z->lp_gradient, (size_t)z->ld * N, &a.g);
+    st.out(z->lk_value, (size_t)N, &a.lk);
+    st.out(z->lk_gradient, (size_t)z->ld * N, &a.dr);
+    if ((rc = st.commit())) return rc;
     int nl = 0;
     if (model->kind == AHMC_MODEL_CALLBACK) {  // user closure, then the metric half of phasepoint
         SplitWork w;
@@ -672,22 +719,13 @@ int ahmc_phasepoint_f64(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metri
 // ---------------------------------------------------------------------------------------------- leapfrog
 static int copy_pp_device(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_phasepoint* a, const ahmc_phasepoint* b,
                           cudaMemcpyKind kind) {
-    auto cp2 = [&](double* dst, const double* src) -> cudaError_t {
-        if (!dst || !src || dst == src) return cudaSuccess;
-        return cudaMemcpy2DAsync(dst, (size_t)b->ld * sizeof(double), src, (size_t)a->ld * sizeof(double),
-                                 (size_t)D * sizeof(double), (size_t)N, kind, ctx->stream);
-    };
-    auto cp1 = [&](double* dst, const double* src) -> cudaError_t {
-        if (!dst || !src || dst == src) return cudaSuccess;
-        return cudaMemcpyAsync(dst, src, (size_t)N * sizeof(double), kind, ctx->stream);
-    };
-    CU(cp2(b->theta, a->theta));
-    CU(cp2(b->r, a->r));
-    CU(cp2(b->lp_gradient, a->lp_gradient));
-    CU(cp2(b->lk_gradient, a->lk_gradient));
-    CU(cp1(b->lp_value, a->lp_value));
-    CU(cp1(b->lk_value, a->lk_value));
-    return AHMC_OK;
+    int rc;
+    if ((rc = copy_cols(ctx, b->theta, b->ld, a->theta, a->ld, D, N, kind))) return rc;
+    if ((rc = copy_cols(ctx, b->r, b->ld, a->r, a->ld, D, N, kind))) return rc;
+    if ((rc = copy_cols(ctx, b->lp_gradient, b->ld, a->lp_gradient, a->ld, D, N, kind))) return rc;
+    if ((rc = copy_cols(ctx, b->lk_gradient, b->ld, a->lk_gradient, a->ld, D, N, kind))) return rc;
+    if ((rc = copy_cols(ctx, b->lp_value, 1, a->lp_value, 1, 1, N, kind))) return rc;
+    return copy_cols(ctx, b->lk_value, 1, a->lk_value, 1, 1, N, kind);
 }
 
 // device alias of a page-locked, device-mapped host pointer (cudaHostAlloc / cudaHostRegister memory under unified
@@ -817,29 +855,18 @@ static int leapfrog_host_pipelined(ahmc_ctx* ctx, const ahmc_model* model, const
 
     // device staging for whatever is not addressed directly
     const int64_t ldi = z_in->ld, ldo = z_out->ld;
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t nMinv = metric_minv_count(metric, D, N);
     const bool stage_in = up != UP_DIRECT, stage_out = !down_direct;
     const bool hasU = metric->kind == AHMC_METRIC_DENSE && metric->cholU;
-    size_t need = (per_chain_minv && !stage_in ? 0 : al(nMinv * 8)) + (hasU ? al((size_t)D * D * 8) : 0);
-    if (stage_in) need += al((size_t)N * 8) + (has_g ? 3 : 2) * al((size_t)ldi * N * 8);
-    if (stage_out) need += 4 * al((size_t)ldo * N * 8) + 2 * al((size_t)N * 8) + 2 * al((size_t)N * 4);
-    if (need > ctx->arena_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        for (int i = 0; i < ahmc_ctx::kPipeStreams; ++i) CU(cudaStreamSynchronize(ctx->pipe[i]));
-        cudaFree(ctx->arena);
-        ctx->arena = nullptr;
-        ctx->arena_bytes = 0;
-        size_t cap = need + need / 4;
-        if (cudaMalloc((void**)&ctx->arena, cap) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for staging failed", cap);
-        ctx->arena_bytes = cap;
-    }
+    size_t need = (per_chain_minv && !stage_in ? 0 : al256(nMinv * 8)) + (hasU ? al256((size_t)D * D * 8) : 0);
+    if (stage_in) need += al256((size_t)N * 8) + (has_g ? 3 : 2) * al256((size_t)ldi * N * 8);
+    if (stage_out) need += 4 * al256((size_t)ldo * N * 8) + 2 * al256((size_t)N * 8) + 2 * al256((size_t)N * 4);
+    if ((rc = grow(ctx, ctx->arena, need, "staging arena", need + need / 4))) return rc;
     size_t off = 0;
     auto carve = [&](bool want, size_t bytes) -> char* {
         if (!want || !bytes) return nullptr;
-        char* p = ctx->arena + off;
-        off += al(bytes);
+        char* p = ctx->arena.p + off;
+        off += al256(bytes);
         return p;
     };
     double* dMinv = (double*)carve(!(per_chain_minv && !stage_in), nMinv * 8);
@@ -1043,66 +1070,50 @@ int ahmc_leapfrog_f64(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric*
                                        status, steps_done, flags);
     Stager st(ctx, host);
     const size_t cin = (size_t)z_in->ld * N, cout = (size_t)z_out->ld * N;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8 * 3);
-    st.reserve(cout * 8 * 4);
-    st.reserve((size_t)N * 8 * 6);
-    if ((rc = st.prepare())) return rc;
     LeapfrogArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D;
     a.N = N;
     a.eps = eps;
-    if ((rc = st.in(eps_chain, (size_t)N, &a.eps_chain))) return rc;
+    st.in(eps_chain, (size_t)N, &a.eps_chain);
     a.n_steps = n_abs;
     a.fwd = n_steps > 0;
     a.temper_alpha = temper_alpha;
     a.ld_in = z_in->ld;
     a.ld_out = z_out->ld;
-    if ((rc = st.in((const double*)z_in->theta, cin, &a.th_in))) return rc;
-    if ((rc = st.in((const double*)z_in->r, cin, &a.r_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_gradient, cin, &a.g_in))) return rc;
-    a.lp_in = nullptr;
-    a.lk_in = nullptr;
-    if ((rc = st.out(z_out->theta, cout, &a.th_out))) return rc;
-    if ((rc = st.out(z_out->r, cout, &a.r_out))) return rc;
-    if ((rc = st.out(z_out->lp_gradient, cout, &a.g_out))) return rc;
-    if ((rc = st.out(z_out->lk_gradient, cout, &a.dr_out))) return rc;
-    if ((rc = st.out(z_out->lp_value, (size_t)N, &a.lp_out))) return rc;
-    if ((rc = st.out(z_out->lk_value, (size_t)N, &a.lk_out))) return rc;
-    if ((rc = st.out(status, (size_t)N, &a.status))) return rc;
-    if ((rc = st.out(steps_done, (size_t)N, &a.steps_done))) return rc;
+    st.in((const double*)z_in->theta, cin, &a.th_in);
+    st.in((const double*)z_in->r, cin, &a.r_in);
+    st.in((const double*)z_in->lp_gradient, cin, &a.g_in);
+    st.out(z_out->theta, cout, &a.th_out);
+    st.out(z_out->r, cout, &a.r_out);
+    st.out(z_out->lp_gradient, cout, &a.g_out);
+    st.out(z_out->lk_gradient, cout, &a.dr_out);
+    st.out(z_out->lp_value, (size_t)N, &a.lp_out);
+    st.out(z_out->lk_value, (size_t)N, &a.lk_out);
+    st.out(status, (size_t)N, &a.status);
+    st.out(steps_done, (size_t)N, &a.steps_done);
+    if ((rc = st.commit())) return rc;
     a.flags = flags;
     const bool compat = flags & AHMC_FLAG_COMPAT_BREAK_ALL;
-    a.min_break = nullptr;
-    a.only_mask = nullptr;
-    {
-        int nl2 = 0;
-        rc = try_dense_trajectory(ctx, model, a, n_abs, eps, temper_alpha, compat, &nl2);
-        if (rc < 0) return rc;
-        if (rc == 1) {
-            ctx->launches += nl2;
-            return finish_call(ctx, st, flags);
-        }
+    if (dense_eligible(model, a.metric, flags, temper_alpha, compat, a.g_in, D)) {
+        int nl = 0;
+        if ((rc = dense_trajectory(ctx, model, a, n_abs, eps, &nl))) return rc;
+        ctx->launches += nl;
+        return finish_call(ctx, st, flags);
     }
     if (model->kind == AHMC_MODEL_CALLBACK) {
         // split-step mode: the work state is the OUTPUT phase point; two small kernels + the user closure per step
         SplitWork w;
         if ((rc = split_workspace(ctx, D, N, z_out->ld, &w))) return rc;
-        auto cp = [&](double* dst, const double* src) -> cudaError_t {
-            if (dst == src) return cudaSuccess;
-            return cudaMemcpy2DAsync(dst, (size_t)a.ld_out * 8, src, (size_t)a.ld_in * 8, (size_t)D * 8, (size_t)N,
-                                     cudaMemcpyDeviceToDevice, ctx->stream);
-        };
-        CU(cp(a.th_out, a.th_in));
-        CU(cp(a.r_out, a.r_in));
-        CU(cp(a.g_out, a.g_in));
-        int nl2 = 0;
+        if ((rc = copy_cols(ctx, a.th_out, a.ld_out, a.th_in, a.ld_in, D, N))) return rc;
+        if ((rc = copy_cols(ctx, a.r_out, a.ld_out, a.r_in, a.ld_in, D, N))) return rc;
+        if ((rc = copy_cols(ctx, a.g_out, a.ld_out, a.g_in, a.ld_in, D, N))) return rc;
+        int nl = 0;
         rc = split_trajectory(ctx, model, a.metric, D, N, eps, a.eps_chain, n_abs, a.fwd, temper_alpha, a.th_out, a.r_out,
                               a.g_out, a.lp_out, a.lk_out, a.dr_out, a.ld_out, a.status ? a.status : w.status,
-                              a.steps_done, w, compat, &nl2);
-        ctx->launches += nl2;
+                              a.steps_done, w, compat, &nl);
+        ctx->launches += nl;
         if (rc) return rc;
         return finish_call(ctx, st, flags);
     }
@@ -1145,18 +1156,15 @@ int ahmc_rand_momentum_f64(ahmc_ctx* ctx, const ahmc_metric* metric, int32_t D, 
     if (N == 0) return AHMC_OK;
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    reserve_metric(st, metric, D, N);
-    st.reserve((size_t)D * N * 8);
-    st.reserve((size_t)ld * N * 8);
-    if ((rc = st.prepare())) return rc;
     MomentumArgs a{};
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D;
     a.N = N;
     a.seed = rng->seed;
     a.offset = rng->offset;
-    if ((rc = st.in(rng->normal_tape, (size_t)D * N, &a.normal_tape))) return rc;
-    if ((rc = st.out(r, (size_t)ld * N, &a.r))) return rc;
+    st.in(rng->normal_tape, (size_t)D * N, &a.normal_tape);
+    st.out(r, (size_t)ld * N, &a.r);
+    if ((rc = st.commit())) return rc;
     a.ld = ld;
     int nl = 0;
     CU(launch_rand_momentum(a, ctx->stream, &nl));
@@ -1165,36 +1173,6 @@ int ahmc_rand_momentum_f64(ahmc_ctx* ctx, const ahmc_metric* metric, int32_t D, 
 }
 
 // ---------------------------------------------------------------------------------------------- transitions
-static int stage_stats(Stager& st, const ahmc_stats* s, int64_t N, StatsDev* d) {
-    memset(d, 0, sizeof *d);
-    if (!s) return AHMC_OK;
-    int rc;
-    if ((rc = st.out(s->n_steps, (size_t)N, &d->n_steps))) return rc;
-    if ((rc = st.out(s->is_accept, (size_t)N, &d->is_accept))) return rc;
-    if ((rc = st.out(s->acceptance_rate, (size_t)N, &d->acceptance_rate))) return rc;
-    if ((rc = st.out(s->log_density, (size_t)N, &d->log_density))) return rc;
-    if ((rc = st.out(s->hamiltonian_energy, (size_t)N, &d->hamiltonian_energy))) return rc;
-    if ((rc = st.out(s->hamiltonian_energy_error, (size_t)N, &d->hamiltonian_energy_error))) return rc;
-    if ((rc = st.out(s->max_hamiltonian_energy_error, (size_t)N, &d->max_hamiltonian_energy_error))) return rc;
-    if ((rc = st.out(s->tree_depth, (size_t)N, &d->tree_depth))) return rc;
-    if ((rc = st.out(s->numerical_error, (size_t)N, &d->numerical_error))) return rc;
-    return AHMC_OK;
-}
-
-static int stage_rng(Stager& st, const ahmc_rng* r, int32_t D, int64_t N, bool nuts, RngDev* d) {
-    d->seed = r->seed;
-    d->offset = r->offset;
-    d->partial_alpha = r->partial_refresh_alpha;
-    d->temper_alpha = r->temper_alpha > 0.0 ? r->temper_alpha : 0.0;
-    d->exp_stride = nuts ? r->exp_stride : 1;
-    d->dir_stride = r->dir_stride;
-    int rc;
-    if ((rc = st.in(r->normal_tape, (size_t)D * N, &d->normal_tape))) return rc;
-    if ((rc = st.in(r->exp_tape, (size_t)(nuts ? r->exp_stride : 1) * N, &d->exp_tape))) return rc;
-    if ((rc = st.in(nuts ? r->dir_tape : (const uint8_t*)nullptr, (size_t)r->dir_stride * N, &d->dir_tape))) return rc;
-    return AHMC_OK;
-}
-
 static int hmc_impl(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* metric, int32_t D, int64_t N,
                     double eps, const double* eps_chain, int32_t n_steps, int32_t n_transitions, const ahmc_rng* rng,
                     const ahmc_phasepoint* z_in, const ahmc_phasepoint* z_out, double* draws, const ahmc_stats* stats,
@@ -1207,151 +1185,85 @@ static int hmc_impl(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* m
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "multi-transition sampling needs a device-resident target");
     if (rng->partial_refresh_alpha != 0.0 && model->kind == AHMC_MODEL_CALLBACK)
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "partial momentum refreshment is not wired into the split-step path");
-    if (!(rng->partial_refresh_alpha > -1.0 && rng->partial_refresh_alpha < 1.0))
-        return fail(ctx, AHMC_ERR_INVALID, "partial_refresh_alpha must be in (-1, 1)");
-    if (!(rng->temper_alpha >= 0.0) || std::isinf(rng->temper_alpha))
-        return fail(ctx, AHMC_ERR_INVALID, "temper_alpha must be 0 (plain Leapfrog) or a finite alpha > 0 (TemperedLeapfrog)");
-    int rc = check_common(ctx, model, metric, D, N);
+    int rc = check_rng_alphas(ctx, rng);
     if (rc) return rc;
+    if ((rc = check_common(ctx, model, metric, D, N))) return rc;
     if ((rc = check_pp(ctx, z_in, D, "z_in", true, N))) return rc;
     if ((rc = check_pp(ctx, z_out, D, "z_out", true, N))) return rc;
     if (n_steps < 1) return fail(ctx, AHMC_ERR_INVALID, "n_steps must be >= 1 (nsteps(tau) = max(1, ...), trajectory.jl:240-243)");
     if (flags & AHMC_FLAG_COMPAT_BREAK_ALL)
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "COMPAT_BREAK_ALL is only available on ahmc_leapfrog_f64");
-    if (metric->kind == AHMC_METRIC_DENSE && !metric->cholU && !(flags & AHMC_FLAG_NO_REFRESH))
-        return fail(ctx, AHMC_ERR_INVALID, "Dense metric needs cholU for the momentum refresh (metric.jl:311-320)");
-    if (z_out->lk_gradient)
-        return fail(ctx, AHMC_ERR_UNSUPPORTED, "transition entry points do not emit lk_gradient; call ahmc_phasepoint_f64 if needed");
+    if ((rc = check_transition_output(ctx, metric, z_out, flags))) return rc;
     if (N == 0) return AHMC_OK;
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    const size_t cin = (size_t)z_in->ld * N, cout = (size_t)z_out->ld * N;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8 * 3);
-    st.reserve(cout * 8 * 3);
-    st.reserve((size_t)D * N * 8);
-    st.reserve((size_t)N * 8 * 16 * n_transitions);
-    if (draws) st.reserve((size_t)D * N * n_transitions * 8);
-    if ((rc = st.prepare())) return rc;
     HmcArgs h{};
     LeapfrogArgs& a = h.lf;
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D;
     a.N = N;
     a.eps = eps;
-    if ((rc = st.in(eps_chain, (size_t)N, &a.eps_chain))) return rc;
+    st.in(eps_chain, (size_t)N, &a.eps_chain);
     a.n_steps = n_steps;
     a.fwd = 1;
     a.temper_alpha = 0.0;
-    a.ld_in = z_in->ld;
-    a.ld_out = z_out->ld;
-    if ((rc = st.in((const double*)z_in->theta, cin, &a.th_in))) return rc;
-    if ((rc = st.in((const double*)z_in->r, cin, &a.r_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_gradient, cin, &a.g_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_value, (size_t)N, &a.lp_in))) return rc;
-    if ((rc = st.out(z_out->theta, cout, &a.th_out))) return rc;
-    if ((rc = st.out(z_out->r, cout, &a.r_out))) return rc;
-    if ((rc = st.out(z_out->lp_gradient, cout, &a.g_out))) return rc;
-    if ((rc = st.out(z_out->lp_value, (size_t)N, &a.lp_out))) return rc;
-    if ((rc = st.out(z_out->lk_value, (size_t)N, &a.lk_out))) return rc;
-    a.dr_out = nullptr;
+    stage_transition_pp(st, z_in, z_out, N, a);
     a.flags = flags;
-    if ((rc = stage_rng(st, rng, D, N, false, &h.rng))) return rc;
-    if ((rc = stage_stats(st, stats, N * n_transitions, &h.st))) return rc;
-    if ((rc = st.out(draws, (size_t)D * N * n_transitions, &h.draws))) return rc;
+    stage_rng(st, rng, D, N, false, &h.rng);
+    stage_stats(st, stats, N * n_transitions, &h.st);
+    st.out(draws, (size_t)D * N * n_transitions, &h.draws);
+    if ((rc = st.commit())) return rc;
     h.n_transitions = n_transitions;
     h.refresh = (flags & AHMC_FLAG_NO_REFRESH) ? 0 : 1;
     int nl = 0;
-    if (model->kind == AHMC_MODEL_CALLBACK) {
-        // refresh -> kinetic energy -> split-step trajectory -> MH select (same semantics as hmc_kernel, unfused)
-        SplitWork w;
-        if ((rc = split_workspace(ctx, D, N, z_out->ld, &w))) return rc;
-        if (h.refresh) {
-            MomentumArgs ma{};
-            ma.metric = a.metric; ma.D = D; ma.N = N; ma.seed = h.rng.seed; ma.offset = h.rng.offset;
-            ma.normal_tape = h.rng.normal_tape; ma.r = w.r0; ma.ld = D;
-            CU(launch_rand_momentum(ma, ctx->stream, &nl));
-        } else {
-            CU(cudaMemcpy2DAsync(w.r0, (size_t)D * 8, a.r_in, (size_t)a.ld_in * 8, (size_t)D * 8, (size_t)N,
-                                 cudaMemcpyDeviceToDevice, ctx->stream));
-        }
-        SplitArgs k0{};  // lk0 = neg kinetic energy of the refreshed momentum
-        k0.metric = a.metric; k0.D = D; k0.N = N; k0.fwd = 1; k0.mul = 1.0; k0.no_kick = 1;
-        k0.r = w.r0; k0.lk = w.lk0; k0.ld = D;
-        CU(launch_kick_energy(k0, ctx->stream, &nl));
-        auto cp = [&](double* dst, const double* src, int64_t lds) -> cudaError_t {
-            if (dst == src) return cudaSuccess;
-            return cudaMemcpy2DAsync(dst, (size_t)a.ld_out * 8, src, (size_t)lds * 8, (size_t)D * 8, (size_t)N,
-                                     cudaMemcpyDeviceToDevice, ctx->stream);
-        };
-        if (a.th_out == a.th_in)
-            return fail(ctx, AHMC_ERR_INVALID, "callback-mode transitions need z_out distinct from z_in (the start point is re-read on rejection)");
-        CU(cp(a.th_out, a.th_in, a.ld_in));
-        CU(cp(a.g_out, a.g_in, a.ld_in));
-        CU(cp(a.r_out, w.r0, D));
-        rc = split_trajectory(ctx, model, a.metric, D, N, eps, a.eps_chain, n_steps, 1, h.rng.temper_alpha, a.th_out, a.r_out, a.g_out,
-                              a.lp_out, a.lk_out, nullptr, a.ld_out, w.status, w.steps, w, false, &nl);
-        if (rc) return rc;
-        MhArgs m{};
-        m.D = D; m.N = N; m.n_steps = n_steps;
-        m.th0 = a.th_in; m.g0 = a.g_in; m.lp0 = a.lp_in; m.ld0 = a.ld_in;
-        m.r0 = w.r0; m.lk0 = w.lk0;
-        m.th = a.th_out; m.r = a.r_out; m.g = a.g_out; m.lp = a.lp_out; m.lk = a.lk_out; m.ld = a.ld_out;
-        m.rng = h.rng; m.st = h.st;
-        CU(launch_mh_select(m, ctx->stream, &nl));
+    // Callback targets, and GEMM-shaped operators of a single plain transition that the tiled K4 trajectory takes, run
+    // unfused with hmc_kernel's semantics: refresh -> kinetic energy -> start point copied to z_out -> trajectory in
+    // place on z_out -> MH select.  Everything else is one fused launch.
+    const bool callback = model->kind == AHMC_MODEL_CALLBACK;
+    const bool k4 = !callback && n_transitions == 1 && a.th_out != a.th_in && h.rng.partial_alpha == 0.0 && !draws &&
+                    dense_eligible(model, a.metric, flags, h.rng.temper_alpha, false, a.g_out, D);
+    if (!callback && !k4) {
+        CU(launch_hmc(h, ctx->stream, &nl));
         ctx->launches += nl;
         return finish_call(ctx, st, flags);
     }
-    if (n_transitions == 1 && a.th_out != a.th_in && h.rng.partial_alpha == 0.0 && !(h.rng.temper_alpha > 0.0) && !draws &&
-        (model->kind == AHMC_MODEL_DENSE_GAUSS || a.metric.kind == AHMC_METRIC_DENSE)) {
-        // GEMM-shaped operators: refresh -> tiled DMMA trajectory (in place on z_out) -> MH select; same semantics as
-        // hmc_kernel.  (Falls through to the fused generic kernel when the tile kernel is not eligible.)
-        SplitWork w;
-        if ((rc = split_workspace(ctx, D, N, z_out->ld, &w))) return rc;
+    if (callback && a.th_out == a.th_in)
+        return fail(ctx, AHMC_ERR_INVALID, "callback-mode transitions need z_out distinct from z_in (the start point is re-read on rejection)");
+    SplitWork w;
+    if ((rc = split_workspace(ctx, D, N, z_out->ld, &w))) return rc;
+    if (h.refresh) {
+        MomentumArgs ma{};
+        ma.metric = a.metric; ma.D = D; ma.N = N; ma.seed = h.rng.seed; ma.offset = h.rng.offset;
+        ma.normal_tape = h.rng.normal_tape; ma.r = w.r0; ma.ld = D;
+        CU(launch_rand_momentum(ma, ctx->stream, &nl));
+    } else if ((rc = copy_cols(ctx, w.r0, D, a.r_in, a.ld_in, D, N))) {
+        return rc;
+    }
+    SplitArgs k0{};  // lk0 = neg kinetic energy of the refreshed momentum
+    k0.metric = a.metric; k0.D = D; k0.N = N; k0.fwd = 1; k0.mul = 1.0; k0.no_kick = 1;
+    k0.r = w.r0; k0.lk = w.lk0; k0.ld = D;
+    CU(launch_kick_energy(k0, ctx->stream, &nl));
+    if ((rc = copy_cols(ctx, a.th_out, a.ld_out, a.th_in, a.ld_in, D, N))) return rc;
+    if ((rc = copy_cols(ctx, a.g_out, a.ld_out, a.g_in, a.ld_in, D, N))) return rc;
+    if ((rc = copy_cols(ctx, a.r_out, a.ld_out, w.r0, D, D, N))) return rc;
+    if (callback) {
+        rc = split_trajectory(ctx, model, a.metric, D, N, eps, a.eps_chain, n_steps, 1, h.rng.temper_alpha, a.th_out, a.r_out,
+                              a.g_out, a.lp_out, a.lk_out, nullptr, a.ld_out, w.status, w.steps, w, false, &nl);
+    } else {
         LeapfrogArgs t = a;
         t.th_in = a.th_out; t.r_in = a.r_out; t.g_in = a.g_out; t.ld_in = a.ld_out;
-        t.status = nullptr; t.steps_done = nullptr; t.only_mask = nullptr; t.min_break = nullptr;
-        const bool gauss = model->kind != AHMC_MODEL_FUNNEL && model->kind != AHMC_MODEL_CALLBACK && model->kind != AHMC_MODEL_USER;
-        const bool metric_ok = a.metric.kind != AHMC_METRIC_DIAG || a.metric.chain_stride == 0;
-        int Dp_, RB_, CB_;
-        if (gauss && metric_ok && !(flags & AHMC_FLAG_EXACT_CHECKS) && dense_tile_shape(D, &Dp_, &RB_, &CB_)) {
-            if (h.refresh) {
-                MomentumArgs ma{};
-                ma.metric = a.metric; ma.D = D; ma.N = N; ma.seed = h.rng.seed; ma.offset = h.rng.offset;
-                ma.normal_tape = h.rng.normal_tape; ma.r = w.r0; ma.ld = D;
-                CU(launch_rand_momentum(ma, ctx->stream, &nl));
-            } else {
-                CU(cudaMemcpy2DAsync(w.r0, (size_t)D * 8, a.r_in, (size_t)a.ld_in * 8, (size_t)D * 8, (size_t)N,
-                                     cudaMemcpyDeviceToDevice, ctx->stream));
-            }
-            SplitArgs k0{};
-            k0.metric = a.metric; k0.D = D; k0.N = N; k0.fwd = 1; k0.mul = 1.0; k0.no_kick = 1;
-            k0.r = w.r0; k0.lk = w.lk0; k0.ld = D;
-            CU(launch_kick_energy(k0, ctx->stream, &nl));
-            auto cp = [&](double* dst, const double* src, int64_t lds) -> cudaError_t {
-                return cudaMemcpy2DAsync(dst, (size_t)a.ld_out * 8, src, (size_t)lds * 8, (size_t)D * 8, (size_t)N,
-                                         cudaMemcpyDeviceToDevice, ctx->stream);
-            };
-            CU(cp(a.th_out, a.th_in, a.ld_in));
-            CU(cp(a.g_out, a.g_in, a.ld_in));
-            CU(cp(a.r_out, w.r0, D));
-            rc = try_dense_trajectory(ctx, model, t, n_steps, eps, 0.0, false, &nl);
-            if (rc < 0) return rc;
-            if (rc == 1) {
-                MhArgs m{};
-                m.D = D; m.N = N; m.n_steps = n_steps;
-                m.th0 = a.th_in; m.g0 = a.g_in; m.lp0 = a.lp_in; m.ld0 = a.ld_in;
-                m.r0 = w.r0; m.lk0 = w.lk0;
-                m.th = a.th_out; m.r = a.r_out; m.g = a.g_out; m.lp = a.lp_out; m.lk = a.lk_out; m.ld = a.ld_out;
-                m.rng = h.rng; m.st = h.st;
-                CU(launch_mh_select(m, ctx->stream, &nl));
-                ctx->launches += nl;
-                return finish_call(ctx, st, flags);
-            }
-        }
+        t.status = nullptr; t.steps_done = nullptr;
+        rc = dense_trajectory(ctx, model, t, n_steps, eps, &nl);
     }
-    CU(launch_hmc(h, ctx->stream, &nl));
+    if (rc) return rc;
+    MhArgs m{};
+    m.D = D; m.N = N; m.n_steps = n_steps;
+    m.th0 = a.th_in; m.g0 = a.g_in; m.lp0 = a.lp_in; m.ld0 = a.ld_in;
+    m.r0 = w.r0; m.lk0 = w.lk0;
+    m.th = a.th_out; m.r = a.r_out; m.g = a.g_out; m.lp = a.lp_out; m.lk = a.lk_out; m.ld = a.ld_out;
+    m.rng = h.rng; m.st = h.st;
+    CU(launch_mh_select(m, ctx->stream, &nl));
     ctx->launches += nl;
     return finish_call(ctx, st, flags);
 }
@@ -1381,12 +1293,9 @@ static int nuts_impl(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* 
     }
     if (n_transitions > 1 && (rng->normal_tape || rng->exp_tape || rng->dir_tape))
         return fail(ctx, AHMC_ERR_INVALID, "random tapes describe ONE transition; multi-transition sampling uses the Philox streams");
-    if (!(rng->partial_refresh_alpha > -1.0 && rng->partial_refresh_alpha < 1.0))
-        return fail(ctx, AHMC_ERR_INVALID, "partial_refresh_alpha must be in (-1, 1)");
-    if (!(rng->temper_alpha >= 0.0) || std::isinf(rng->temper_alpha))
-        return fail(ctx, AHMC_ERR_INVALID, "temper_alpha must be 0 (plain Leapfrog) or a finite alpha > 0 (TemperedLeapfrog)");
-    int rc = check_common(ctx, model, metric, D, N);
+    int rc = check_rng_alphas(ctx, rng);
     if (rc) return rc;
+    if ((rc = check_common(ctx, model, metric, D, N))) return rc;
     if ((rc = check_pp(ctx, z_in, D, "z_in", true, N))) return rc;
     if ((rc = check_pp(ctx, z_out, D, "z_out", true, N))) return rc;
     if (max_depth < 0 || max_depth > 20) return fail(ctx, AHMC_ERR_INVALID, "max_depth must be in 0..20");
@@ -1398,53 +1307,40 @@ static int nuts_impl(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* 
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "NUTS needs a device-resident target: callback (split-step) models are supported by ahmc_leapfrog_f64 / ahmc_hmc_transition_f64 / ahmc_phasepoint_f64 only; express the target as CUDA source (ahmc_model_create_user) to run NUTS on it");
     if (model->kind == AHMC_MODEL_USER && (cfg || (flags & (AHMC_FLAG_NUTS_SLICE_TS | AHMC_FLAG_NUTS_CLASSIC | AHMC_FLAG_NUTS_STRICT))))
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "run-time compiled targets: MultinomialTS + GeneralisedNoUTurn without in-launch adaptation");
-    if (metric->kind == AHMC_METRIC_DENSE && !metric->cholU && !(flags & AHMC_FLAG_NO_REFRESH))
-        return fail(ctx, AHMC_ERR_INVALID, "Dense metric needs cholU for the momentum refresh (metric.jl:311-320)");
-    if (z_out->lk_gradient)
-        return fail(ctx, AHMC_ERR_UNSUPPORTED, "transition entry points do not emit lk_gradient; call ahmc_phasepoint_f64 if needed");
+    if ((rc = check_transition_output(ctx, metric, z_out, flags))) return rc;
     if (rng->exp_tape && rng->exp_stride < 1) return fail(ctx, AHMC_ERR_INVALID, "exp_tape needs exp_stride >= 1");
     if (rng->dir_tape && rng->dir_stride < max_depth) return fail(ctx, AHMC_ERR_INVALID, "dir_tape needs dir_stride >= max_depth");
     if (N == 0) return AHMC_OK;
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    const size_t cin = (size_t)z_in->ld * N, cout = (size_t)z_out->ld * N;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8 * 3);
-    st.reserve(cout * 8 * 3);
-    st.reserve((size_t)D * N * 8);
-    st.reserve((size_t)N * 8 * 16 * n_transitions);
-    if (draws) st.reserve((size_t)D * N * n_transitions * 8);
-    if (rng->exp_tape) st.reserve((size_t)rng->exp_stride * N * 8);
-    if (rng->dir_tape) st.reserve((size_t)rng->dir_stride * N);
-    if (cfg) {
-        st.reserve((size_t)N * 8);
-        if (cfg->Minv_chain) st.reserve((size_t)N * D * 8);
-        if (cfg->eps_trace) st.reserve((size_t)N * n_transitions * 8);
-    }
-    if ((rc = st.prepare())) return rc;
     NutsArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
+    if (cfg) {
+        st.inout(cfg->eps_chain, (size_t)N, &a.ad.eps);
+        st.out(cfg->Minv_chain, (size_t)N * D, &a.ad.minv);
+        st.out(cfg->eps_trace, (size_t)N * n_transitions, &a.ad.eps_trace);
+    } else {
+        st.in(eps_chain, (size_t)N, &a.eps_chain);
+    }
+    stage_transition_pp(st, z_in, z_out, N, a);
+    stage_rng(st, rng, D, N, true, &a.rng);
+    stage_stats(st, stats, N * n_transitions, &a.st);
+    st.out(draws, (size_t)D * N * n_transitions, &a.draws);
+    if ((rc = st.commit())) return rc;
     int n_prep = 0;
     if (a.metric.kind == AHMC_METRIC_DENSE && D > 16 && D <= 512) {
         // the cooperative form streams Minv / cholU in chunks of columns: hand it copies whose columns are padded to the
         // shared-memory leading dimension, so that a chunk is one bulk copy (two small kernels per call, on the stream)
         const size_t per = coop_padded_doubles(D);
-        if (2 * per > ctx->coop_scratch_doubles) {
-            CU(cudaStreamSynchronize(ctx->stream));
-            cudaFree(ctx->coop_scratch);
-            ctx->coop_scratch = nullptr;
-            ctx->coop_scratch_doubles = 0;
-            if (cudaMalloc((void**)&ctx->coop_scratch, 2 * per * sizeof(double)) != cudaSuccess)
-                return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc for the column-padded metric failed");
-            ctx->coop_scratch_doubles = 2 * per;
-        }
-        CU(launch_pad_columns(a.metric.Minv, D, ctx->coop_scratch, ctx->stream));
-        a.metric.Minv_coop = ctx->coop_scratch;
+        if ((rc = grow(ctx, ctx->coop_scratch, 2 * per * sizeof(double), "column-padded metric"))) return rc;
+        double* coop = (double*)ctx->coop_scratch.p;
+        CU(launch_pad_columns(a.metric.Minv, D, coop, ctx->stream));
+        a.metric.Minv_coop = coop;
         ++n_prep;
         if (a.metric.cholU) {
-            CU(launch_pad_columns(a.metric.cholU, D, ctx->coop_scratch + per, ctx->stream));
-            a.metric.cholU_coop = ctx->coop_scratch + per;
+            CU(launch_pad_columns(a.metric.cholU, D, coop + per, ctx->stream));
+            a.metric.cholU_coop = coop + per;
             ++n_prep;
         }
     }
@@ -1465,47 +1361,18 @@ static int nuts_impl(ahmc_ctx* ctx, const ahmc_model* model, const ahmc_metric* 
         if (!stan_window_schedule(ad, cfg->init_buffer, cfg->term_buffer, cfg->window_size, cfg->n_adapts))
             return fail(ctx, AHMC_ERR_UNSUPPORTED, "the window schedule (stan_adaptor.jl:13-50) needs more than %d splits",
                         (int)(sizeof(ad.splits) / sizeof(ad.splits[0])));
-        if ((rc = st.inout(cfg->eps_chain, (size_t)N, &ad.eps))) return rc;
         a.eps_chain = ad.eps;
-        if ((rc = st.out(cfg->Minv_chain, (size_t)N * D, &ad.minv))) return rc;
-        if ((rc = st.out(cfg->eps_trace, (size_t)N * n_transitions, &ad.eps_trace))) return rc;
-    } else if ((rc = st.in(eps_chain, (size_t)N, &a.eps_chain))) {
-        return rc;
     }
     a.max_depth = max_depth;
     a.delta_max = delta_max;
     a.sampler = (flags & AHMC_FLAG_NUTS_SLICE_TS) ? 1 : 0;
     a.criterion = (flags & AHMC_FLAG_NUTS_STRICT) ? 2 : (flags & AHMC_FLAG_NUTS_CLASSIC) ? 1 : 0;
     a.refresh = (flags & AHMC_FLAG_NO_REFRESH) ? 0 : 1;
-    a.ld_in = z_in->ld;
-    a.ld_out = z_out->ld;
-    if ((rc = st.in((const double*)z_in->theta, cin, &a.th_in))) return rc;
-    if ((rc = st.in((const double*)z_in->r, cin, &a.r_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_gradient, cin, &a.g_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_value, (size_t)N, &a.lp_in))) return rc;
-    if ((rc = st.out(z_out->theta, cout, &a.th_out))) return rc;
-    if ((rc = st.out(z_out->r, cout, &a.r_out))) return rc;
-    if ((rc = st.out(z_out->lp_gradient, cout, &a.g_out))) return rc;
-    if ((rc = st.out(z_out->lp_value, (size_t)N, &a.lp_out))) return rc;
-    if ((rc = st.out(z_out->lk_value, (size_t)N, &a.lk_out))) return rc;
-    a.dr_out = nullptr;
-    if ((rc = stage_rng(st, rng, D, N, true, &a.rng))) return rc;
-    if ((rc = stage_stats(st, stats, N * n_transitions, &a.st))) return rc;
-    if ((rc = st.out(draws, (size_t)D * N * n_transitions, &a.draws))) return rc;
     a.n_transitions = n_transitions;
     // per-chain tree workspace
     a.scratch_stride = nuts_scratch_doubles_per_chain(D, max_depth, cfg != nullptr);
-    size_t need = (size_t)a.scratch_stride * (size_t)N * sizeof(double);
-    if (need > ctx->nuts_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->nuts_scratch);
-        ctx->nuts_scratch = nullptr;
-        ctx->nuts_scratch_bytes = 0;
-        cudaError_t e = cudaMalloc((void**)&ctx->nuts_scratch, need);
-        if (e != cudaSuccess) return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the NUTS workspace failed: %s", need, cudaGetErrorString(e));
-        ctx->nuts_scratch_bytes = need;
-    }
-    a.scratch = ctx->nuts_scratch;
+    if ((rc = grow(ctx, ctx->nuts_scratch, (size_t)a.scratch_stride * (size_t)N * sizeof(double), "NUTS workspace"))) return rc;
+    a.scratch = (double*)ctx->nuts_scratch.p;
     int nl = 0;
     CU(launch_nuts(a, ctx->stream, &nl));
     ctx->launches += nl;
@@ -1529,28 +1396,24 @@ int ahmc_leapfrog_trajectory_f64(ahmc_ctx* ctx, const ahmc_model* model, const a
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
     const size_t cin = (size_t)z_in->ld * N, ctraj = (size_t)step_stride * n_abs;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8 * 3);
-    st.reserve(ctraj * 8 * 4);
-    st.reserve((size_t)N * n_abs * 8 * 2 + (size_t)N * 16);
-    if ((rc = st.prepare())) return rc;
     TrajArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D; a.N = N; a.eps = eps;
-    if ((rc = st.in(eps_chain, (size_t)N, &a.eps_chain))) return rc;
+    st.in(eps_chain, (size_t)N, &a.eps_chain);
     a.n_steps = n_abs; a.fwd = n_steps > 0; a.temper_alpha = temper_alpha;
     a.ld_in = z_in->ld; a.ld_out = traj->ld; a.step_stride = step_stride;
-    if ((rc = st.in((const double*)z_in->theta, cin, &a.th_in))) return rc;
-    if ((rc = st.in((const double*)z_in->r, cin, &a.r_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_gradient, cin, &a.g_in))) return rc;
-    if ((rc = st.out(traj->theta, ctraj, &a.th_out))) return rc;
-    if ((rc = st.out(traj->r, ctraj, &a.r_out))) return rc;
-    if ((rc = st.out(traj->lp_gradient, ctraj, &a.g_out))) return rc;
-    if ((rc = st.out(traj->lk_gradient, ctraj, &a.dr_out))) return rc;
-    if ((rc = st.out(traj->lp_value, (size_t)N * n_abs, &a.lp_out))) return rc;
-    if ((rc = st.out(traj->lk_value, (size_t)N * n_abs, &a.lk_out))) return rc;
-    if ((rc = st.out(steps_done, (size_t)N, &a.steps_done))) return rc;
+    st.in((const double*)z_in->theta, cin, &a.th_in);
+    st.in((const double*)z_in->r, cin, &a.r_in);
+    st.in((const double*)z_in->lp_gradient, cin, &a.g_in);
+    st.out(traj->theta, ctraj, &a.th_out);
+    st.out(traj->r, ctraj, &a.r_out);
+    st.out(traj->lp_gradient, ctraj, &a.g_out);
+    st.out(traj->lk_gradient, ctraj, &a.dr_out);
+    st.out(traj->lp_value, (size_t)N * n_abs, &a.lp_out);
+    st.out(traj->lk_value, (size_t)N * n_abs, &a.lk_out);
+    st.out(steps_done, (size_t)N, &a.steps_done);
+    if ((rc = st.commit())) return rc;
     int nl = 0;
     CU(launch_trajectory(a, ctx->stream, &nl));
     ctx->launches += nl;
@@ -1570,54 +1433,24 @@ int ahmc_hmc_multinomial_transition_f64(ahmc_ctx* ctx, const ahmc_model* model, 
         return fail(ctx, AHMC_ERR_INVALID, "need n_steps >= 1 and 0 <= n_steps_fwd <= n_steps (rand(0:n_steps), trajectory.jl:373)");
     if (model->kind == AHMC_MODEL_CALLBACK || model->kind == AHMC_MODEL_USER)
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "MultinomialTS static transitions: built-in targets only");
-    if (metric->kind == AHMC_METRIC_DENSE && !metric->cholU && !(flags & AHMC_FLAG_NO_REFRESH))
-        return fail(ctx, AHMC_ERR_INVALID, "Dense metric needs cholU for the momentum refresh (metric.jl:311-320)");
-    if (z_out->lk_gradient)
-        return fail(ctx, AHMC_ERR_UNSUPPORTED, "transition entry points do not emit lk_gradient; call ahmc_phasepoint_f64 if needed");
-    if (!(rng->partial_refresh_alpha > -1.0 && rng->partial_refresh_alpha < 1.0))
-        return fail(ctx, AHMC_ERR_INVALID, "partial_refresh_alpha must be in (-1, 1)");
-    if (!(rng->temper_alpha >= 0.0) || std::isinf(rng->temper_alpha))
-        return fail(ctx, AHMC_ERR_INVALID, "temper_alpha must be 0 (plain Leapfrog) or a finite alpha > 0 (TemperedLeapfrog)");
+    if ((rc = check_transition_output(ctx, metric, z_out, flags))) return rc;
+    if ((rc = check_rng_alphas(ctx, rng))) return rc;
     if (N == 0) return AHMC_OK;
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    const size_t cin = (size_t)z_in->ld * N, cout = (size_t)z_out->ld * N;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8 * 3);
-    st.reserve(cout * 8 * 3);
-    st.reserve((size_t)D * N * 8);
-    st.reserve((size_t)N * 8 * 16);
-    if ((rc = st.prepare())) return rc;
     MultinomialArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D; a.N = N; a.eps = eps;
-    if ((rc = st.in(eps_chain, (size_t)N, &a.eps_chain))) return rc;
+    st.in(eps_chain, (size_t)N, &a.eps_chain);
     a.n_steps = n_steps; a.n_fwd = n_steps_fwd;
     a.refresh = (flags & AHMC_FLAG_NO_REFRESH) ? 0 : 1;
-    a.ld_in = z_in->ld; a.ld_out = z_out->ld;
-    if ((rc = st.in((const double*)z_in->theta, cin, &a.th_in))) return rc;
-    if ((rc = st.in((const double*)z_in->r, cin, &a.r_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_gradient, cin, &a.g_in))) return rc;
-    if ((rc = st.in((const double*)z_in->lp_value, (size_t)N, &a.lp_in))) return rc;
-    if ((rc = st.out(z_out->theta, cout, &a.th_out))) return rc;
-    if ((rc = st.out(z_out->r, cout, &a.r_out))) return rc;
-    if ((rc = st.out(z_out->lp_gradient, cout, &a.g_out))) return rc;
-    if ((rc = st.out(z_out->lp_value, (size_t)N, &a.lp_out))) return rc;
-    if ((rc = st.out(z_out->lk_value, (size_t)N, &a.lk_out))) return rc;
-    if ((rc = stage_rng(st, rng, D, N, false, &a.rng))) return rc;
-    if ((rc = stage_stats(st, stats, N, &a.st))) return rc;
-    const size_t need = (size_t)(n_steps + 1) * (size_t)N * sizeof(double);
-    if (need > ctx->mn_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->mn_scratch);
-        ctx->mn_scratch = nullptr;
-        ctx->mn_scratch_bytes = 0;
-        if (cudaMalloc((void**)&ctx->mn_scratch, need) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the multinomial energy tape failed", need);
-        ctx->mn_scratch_bytes = need;
-    }
-    a.energies = ctx->mn_scratch;
+    stage_transition_pp(st, z_in, z_out, N, a);
+    stage_rng(st, rng, D, N, false, &a.rng);
+    stage_stats(st, stats, N, &a.st);
+    if ((rc = st.commit())) return rc;
+    if ((rc = grow(ctx, ctx->mn_scratch, (size_t)(n_steps + 1) * (size_t)N * sizeof(double), "multinomial energy tape"))) return rc;
+    a.energies = (double*)ctx->mn_scratch.p;
     int nl = 0;
     CU(launch_multinomial(a, ctx->stream, &nl));
     ctx->launches += nl;
@@ -1669,34 +1502,19 @@ int ahmc_adapt_summary_f64(ahmc_ctx* ctx, int32_t D, int64_t N, const double* th
     if (!ctx || !theta || !out) return fail(ctx, AHMC_ERR_INVALID, "NULL ctx/theta/out");
     if (D < 1 || N < 1 || ld < D) return fail(ctx, AHMC_ERR_INVALID, "need D >= 1, N >= 1, ld >= D");
     DeviceGuard g(ctx->device);
-    const int blocks = (int)(N < 148 ? N : 148);
-    const size_t need = ((size_t)blocks * (D + 1) + 2) * sizeof(double);
-    if (need > ctx->adapt_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->adapt_scratch);
-        ctx->adapt_scratch = nullptr;
-        ctx->adapt_scratch_bytes = 0;
-        if (cudaMalloc((void**)&ctx->adapt_scratch, need) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the adaptor workspace failed", need);
-        ctx->adapt_scratch_bytes = need;
-        CU(cudaMemsetAsync(ctx->adapt_scratch, 0, need, ctx->stream));
-    }
-    Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    st.reserve((size_t)ld * N * 8);
-    st.reserve((size_t)N * 8);
-    st.reserve((size_t)(2 + 2 * D) * 8);
-    int rc = st.prepare();
+    int blocks;
+    int rc = adapt_workspace(ctx, D, N, &blocks);
     if (rc) return rc;
+    Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
     const double *d_theta, *d_alpha;
     double* d_out;
-    if ((rc = st.in(theta, (size_t)ld * N, &d_theta))) return rc;
-    if ((rc = st.in(acceptance_rate, (size_t)N, &d_alpha))) return rc;
-    if ((rc = st.out(out, (size_t)(2 + 2 * D), &d_out))) return rc;
-    // workspace: [counter (as 2 doubles)] [partials]
-    unsigned* counter = (unsigned*)ctx->adapt_scratch;
-    double* partial = ctx->adapt_scratch + 2;
+    st.in(theta, (size_t)ld * N, &d_theta);
+    st.in(acceptance_rate, (size_t)N, &d_alpha);
+    st.out(out, (size_t)(2 + 2 * D), &d_out);
+    if ((rc = st.commit())) return rc;
+    double* ws = (double*)ctx->adapt_scratch.p;
     int nl = 0;
-    CU(launch_adapt_summary(D, N, d_theta, ld, d_alpha, d_out, partial, counter, blocks, ctx->stream, &nl));
+    CU(launch_adapt_summary(D, N, d_theta, ld, d_alpha, d_out, ws + 2, (unsigned*)ws, blocks, ctx->stream, &nl));
     ctx->launches += nl;
     return finish_call(ctx, st, flags);
 }
@@ -1707,16 +1525,13 @@ int ahmc_adapt_cov_f64(ahmc_ctx* ctx, int32_t D, int64_t N, const double* theta,
     if (D < 1 || N < 1 || ld < D) return fail(ctx, AHMC_ERR_INVALID, "need D >= 1, N >= 1, ld >= D");
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
-    st.reserve((size_t)ld * N * 8);
-    st.reserve((size_t)D * 8);
-    st.reserve((size_t)D * D * 8);
-    int rc = st.prepare();
-    if (rc) return rc;
     const double *d_theta, *d_mean;
     double* d_out;
-    if ((rc = st.in(theta, (size_t)ld * N, &d_theta))) return rc;
-    if ((rc = st.in(mean, (size_t)D, &d_mean))) return rc;
-    if ((rc = st.out(out, (size_t)D * D, &d_out))) return rc;
+    st.in(theta, (size_t)ld * N, &d_theta);
+    st.in(mean, (size_t)D, &d_mean);
+    st.out(out, (size_t)D * D, &d_out);
+    int rc = st.commit();
+    if (rc) return rc;
     int nl = 0;
     CU(launch_adapt_cov(D, N, d_theta, ld, d_mean, d_out, ctx->stream, &nl));
     ctx->launches += nl;
@@ -1739,26 +1554,23 @@ int ahmc_find_good_stepsize_f64(ahmc_ctx* ctx, const ahmc_model* model, const ah
     DeviceGuard g(ctx->device);
     Stager st(ctx, flags & AHMC_FLAG_HOST_BUFFERS);
     const size_t cin = (size_t)z->ld * N;
-    reserve_metric(st, metric, D, N);
-    st.reserve(cin * 8); st.reserve(cin * 8); st.reserve(cin * 8); st.reserve((size_t)D * N * 8);
-    st.reserve((size_t)N * 8); st.reserve((size_t)N * 8);
-    if ((rc = st.prepare())) return rc;
     FindEpsArgs a{};
     a.model = model_dev(model);
-    if ((rc = stage_metric(st, metric, D, N, &a.metric))) return rc;
+    stage_metric(st, metric, D, N, &a.metric);
     a.D = D;
     a.N = N;
     a.ld = z->ld;
-    if ((rc = st.in((const double*)z->theta, cin, &a.th))) return rc;
-    if ((rc = st.in((const double*)z->lp_gradient, cin, &a.g))) return rc;
-    if ((rc = st.in((const double*)z->lp_value, (size_t)N, &a.lp))) return rc;
-    if ((rc = st.in(rng->normal_tape, (size_t)D * N, &a.normal_tape))) return rc;
+    st.in((const double*)z->theta, cin, &a.th);
+    st.in((const double*)z->lp_gradient, cin, &a.g);
+    st.in((const double*)z->lp_value, (size_t)N, &a.lp);
+    st.in(rng->normal_tape, (size_t)D * N, &a.normal_tape);
     a.seed = rng->seed;
     a.offset = rng->offset;
     a.eps0 = initial_step_size;
     a.max_iters = max_n_iters;
-    if ((rc = st.out(eps_out, (size_t)N, &a.eps_out))) return rc;
-    if ((rc = st.out(r_out, cin, &a.r_out))) return rc;
+    st.out(eps_out, (size_t)N, &a.eps_out);
+    st.out(r_out, cin, &a.r_out);
+    if ((rc = st.commit())) return rc;
     int nl = 0;
     CU(launch_find_eps(a, ctx->stream, &nl));
     ctx->launches += nl;
@@ -1774,11 +1586,10 @@ struct ahmc_comm {
 struct ahmc_pooled {
     int D = 0;
     int64_t N = 0;
-    char* dev = nullptr;  // one allocation: state | record | gathered (grown on demand) ...
+    char* dev = nullptr;  // one allocation: state | eps_chain | minv | w_mu | w_M2 | record | merged
     void* state = nullptr;
     double *eps_chain = nullptr, *minv = nullptr, *w_mu = nullptr, *w_M2 = nullptr, *record = nullptr, *merged = nullptr;
-    double* gathered = nullptr;
-    int gathered_ranks = 0;
+    DevBuf gathered;  // R records of the last multi-rank exchange (grown on demand)
 };
 
 int ahmc_comm_unique_id(ahmc_ctx* ctx, void* id128_out) {
@@ -1848,20 +1659,19 @@ int ahmc_pooled_create(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cf
     if (!a) return fail(ctx, AHMC_ERR_NOMEM, "out of host memory");
     a->D = D;
     a->N = N;
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t rec = (size_t)(2 + 2 * D) * 8;
-    const size_t total = al(pooled_state_bytes()) + al((size_t)N * 8) + 3 * al((size_t)D * 8) + 2 * al(rec);
+    const size_t total = al256(pooled_state_bytes()) + al256((size_t)N * 8) + 3 * al256((size_t)D * 8) + 2 * al256(rec);
     if (cudaMalloc((void**)&a->dev, total) != cudaSuccess) {
         delete a;
         return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the pooled adaptor failed", total);
     }
     char* p = a->dev;
-    a->state = p; p += al(pooled_state_bytes());
-    a->eps_chain = (double*)p; p += al((size_t)N * 8);
-    a->minv = (double*)p; p += al((size_t)D * 8);
-    a->w_mu = (double*)p; p += al((size_t)D * 8);
-    a->w_M2 = (double*)p; p += al((size_t)D * 8);
-    a->record = (double*)p; p += al(rec);
+    a->state = p; p += al256(pooled_state_bytes());
+    a->eps_chain = (double*)p; p += al256((size_t)N * 8);
+    a->minv = (double*)p; p += al256((size_t)D * 8);
+    a->w_mu = (double*)p; p += al256((size_t)D * 8);
+    a->w_M2 = (double*)p; p += al256((size_t)D * 8);
+    a->record = (double*)p; p += al256(rec);
     a->merged = (double*)p;
     std::vector<char> img(pooled_state_bytes());
     pooled_state_init(img.data(), cfg->eps0, sched, cfg->delta, cfg->gamma, cfg->t0, cfg->kappa, cfg->n_adapts,
@@ -1883,7 +1693,7 @@ int ahmc_pooled_destroy(ahmc_ctx* ctx, ahmc_pooled* a) {
     DeviceGuard g(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     cudaFree(a->dev);
-    cudaFree(a->gathered);
+    cudaFree(a->gathered.p);
     delete a;
     return AHMC_OK;
 }
@@ -1898,35 +1708,19 @@ int ahmc_adapt_exchange_f64(ahmc_ctx* ctx, ahmc_comm* comm, ahmc_pooled* a, int3
     DeviceGuard g(ctx->device);
     const int R = comm ? comm->nranks : 1;
     const size_t rec = (size_t)(2 + 2 * D);
-    if (R > 1 && a->gathered_ranks < R) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(a->gathered);
-        a->gathered = nullptr;
-        if (cudaMalloc((void**)&a->gathered, rec * 8 * (size_t)R) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc for the gathered records failed");
-        a->gathered_ranks = R;
-    }
-    // K5: this rank's record (same workspace discipline as ahmc_adapt_summary_f64)
-    const int blocks = (int)(N < 148 ? N : 148);
-    const size_t need = ((size_t)blocks * (D + 1) + 2) * sizeof(double);
-    if (need > ctx->adapt_scratch_bytes) {
-        CU(cudaStreamSynchronize(ctx->stream));
-        cudaFree(ctx->adapt_scratch);
-        ctx->adapt_scratch = nullptr;
-        ctx->adapt_scratch_bytes = 0;
-        if (cudaMalloc((void**)&ctx->adapt_scratch, need) != cudaSuccess)
-            return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the adaptor workspace failed", need);
-        ctx->adapt_scratch_bytes = need;
-        CU(cudaMemsetAsync(ctx->adapt_scratch, 0, need, ctx->stream));
-    }
+    int rc;
+    if (R > 1 && (rc = grow(ctx, a->gathered, rec * 8 * (size_t)R, "gathered records"))) return rc;
+    // K5: this rank's record
+    int blocks;
+    if ((rc = adapt_workspace(ctx, D, N, &blocks))) return rc;
+    double* ws = (double*)ctx->adapt_scratch.p;
     int nl = 0;
-    CU(launch_adapt_summary(D, N, theta, ld, acceptance_rate, a->record, ctx->adapt_scratch + 2, (unsigned*)ctx->adapt_scratch,
-                            blocks, ctx->stream, &nl));
+    CU(launch_adapt_summary(D, N, theta, ld, acceptance_rate, a->record, ws + 2, (unsigned*)ws, blocks, ctx->stream, &nl));
     const double* gathered = a->record;
     if (R > 1) {
-        int rc = nccl_allgather_f64(a->record, a->gathered, rec, comm->nccl, ctx->stream);
-        if (rc) return fail(ctx, AHMC_ERR_CUDA, "ncclAllGather: %s", nccl_err(rc));
-        gathered = a->gathered;
+        if ((rc = nccl_allgather_f64(a->record, (double*)a->gathered.p, rec, comm->nccl, ctx->stream)))
+            return fail(ctx, AHMC_ERR_CUDA, "ncclAllGather: %s", nccl_err(rc));
+        gathered = (double*)a->gathered.p;
     }
     CU(launch_pooled_update(a->state, gathered, R, D, a->w_mu, a->w_M2, a->minv, a->eps_chain, N, eps_trace, a->merged,
                             ctx->stream, &nl));

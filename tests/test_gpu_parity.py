@@ -710,7 +710,7 @@ def test_small_host_buffer_calls_first_on_a_fresh_context_stay_inside_the_stagin
     """ADVICE r1 (high): the staging arena was sized from grouped reservations while every staged array is rounded up to
     256 B on its own, so N = 1 / small-D host calls made FIRST in a process wrote past the arena.  A fresh interpreter makes
     them first (phasepoint, step, static transition, NUTS) under compute-sanitizer-free conditions by checking results
-    against device calls; the arena now carries slack for the roundings and alloc() fails instead of overrunning."""
+    against device calls; the arena is now sized from the very arrays a call stages, each rounded up on its own."""
     import subprocess, sys, os
     code = r'''
 import numpy as np, torch, ahmc_b200 as A
