@@ -114,6 +114,9 @@ PROTOTYPES = {
     "ahmc_pooled_minv": (_vp, [_vp]),
     "ahmc_adapt_exchange_f64": (C.c_int, [_vp, _vp, _vp, C.c_int32, C.c_int64, _vp, C.c_int64, _vp, _vp, C.c_uint32]),
     "ahmc_pooled_state": (C.c_int, [_vp, _vp, _dp, _dp, C.POINTER(C.c_int32), _dp]),
+    "ahmc_pooled_create_dense": (C.c_int, [_vp, C.c_int32, C.c_int64, C.POINTER(PooledCfg), _dp, C.POINTER(_vp)]),
+    "ahmc_pooled_cholu": (_vp, [_vp]),
+    "ahmc_pooled_state_dense": (C.c_int, [_vp, _vp, _dp, _dp, _dp, C.POINTER(C.c_int32), _dp, C.POINTER(C.c_int32)]),
 }
 
 _lib = None

@@ -483,11 +483,14 @@ class Comm:
 class PooledDeviceAdaptor:
     """`ahmc_pooled`: StanHMCAdaptor(WelfordVar, NesterovDualAveraging) pooled over all chains of all ranks, resident on
     the device.  `eps` (N,) and `Minv` (D,) are torch views of the buffers the library updates in place -- hand them to
-    `Leapfrog` / `DiagEuclideanMetric` once; `exchange` then needs no host work beyond one foreign call."""
+    `Leapfrog` / `DiagEuclideanMetric` once; `exchange` then needs no host work beyond one foreign call.
+    `dense=True`: StanHMCAdaptor(WelfordCov, ...) (ahmc_pooled_create_dense, D <= 512); `Minv0` is (D, D), `Minv` and `cholU`
+    (the upper factor U, U'U = Minv) are (D, D) views of the column-major device buffers -- hand them to
+    `DenseEuclideanMetric(ad.Minv, cholU=ad.cholU)` once."""
 
     def __init__(self, device: int, D: int, N: int, n_adapts: int, eps0: float, delta: float = 0.8, adapt_metric: bool = True,
                  init_buffer: int = 75, term_buffer: int = 50, window_size: int = 25, gamma: float = 0.05, t0: float = 10.0,
-                 kappa: float = 0.75, n_min: int = 10, Minv0=None):
+                 kappa: float = 0.75, n_min: int = 10, Minv0=None, dense: bool = False):
         import ctypes as C
 
         import torch
@@ -495,16 +498,24 @@ class PooledDeviceAdaptor:
         from . import _lib as L
 
         self.ctx = ctx = A.get_context(device)
-        self.D, self.N, self.n_adapts = D, N, n_adapts
+        self.D, self.N, self.n_adapts, self.dense = D, N, n_adapts, dense
         cfg = L.PooledCfg(n_adapts, init_buffer, term_buffer, window_size, delta, gamma, t0, kappa, float(eps0),
                           1 if adapt_metric else 0, n_min)
         m0 = None if Minv0 is None else np.ascontiguousarray(Minv0, dtype=np.float64)
+        if dense and m0 is not None:
+            if m0.shape != (D, D):
+                raise L.InvalidArgument(L.ERR_INVALID, f"Minv0 must be ({D}, {D}), got {m0.shape}")
+            m0 = np.ascontiguousarray(m0.T)  # column-major
         self.h = C.c_void_p()
-        ctx.check(ctx.lib.ahmc_pooled_create(ctx.h, D, N, C.byref(cfg), None if m0 is None else m0.ctypes.data_as(L._dp),
-                                             C.byref(self.h)))
+        create = ctx.lib.ahmc_pooled_create_dense if dense else ctx.lib.ahmc_pooled_create
+        ctx.check(create(ctx.h, D, N, C.byref(cfg), None if m0 is None else m0.ctypes.data_as(L._dp), C.byref(self.h)))
         dev = torch.device("cuda", device)
         self.eps = torch.as_tensor(A._RawCuda(ctx.lib.ahmc_pooled_eps(self.h), (N,)), device=dev)
-        self.Minv = torch.as_tensor(A._RawCuda(ctx.lib.ahmc_pooled_minv(self.h), (D,)), device=dev)
+        if dense:  # a row-major (D, D) view of a column-major buffer is the transpose: present the logical matrices
+            self.Minv = torch.as_tensor(A._RawCuda(ctx.lib.ahmc_pooled_minv(self.h), (D, D)), device=dev).T
+            self.cholU = torch.as_tensor(A._RawCuda(ctx.lib.ahmc_pooled_cholu(self.h), (D, D)), device=dev).T
+        else:
+            self.Minv = torch.as_tensor(A._RawCuda(ctx.lib.ahmc_pooled_minv(self.h), (D,)), device=dev)
 
     def exchange(self, theta, acceptance_rate, comm: Optional[Comm] = None, eps_trace=None, flags: int = A.L.FLAG_ASYNC):
         """`adapt!` of the next iteration (ahmc_adapt_exchange_f64): K5 -> all-gather -> merge + adaptor update, on the stream"""
@@ -513,12 +524,22 @@ class PooledDeviceAdaptor:
                                                              None if eps_trace is None else eps_trace.data_ptr(), flags))
 
     def state(self):
-        """synchronising read-back -> dict(eps, Minv, iteration, merged_record)"""
+        """synchronising read-back -> dict(eps, Minv, iteration, merged_record); a dense adaptor adds cholU (U) and
+        failed_iteration (the first iteration whose estimate was not positive definite, 0 = none)"""
         import ctypes as C
 
         from . import _lib as L
 
         eps, it = C.c_double(), C.c_int32()
+        if self.dense:
+            D = self.D
+            failed = C.c_int32()
+            minv, U, rec = np.empty((D, D)), np.empty((D, D)), np.empty(2 + 2 * D + D * D)
+            self.ctx.check(self.ctx.lib.ahmc_pooled_state_dense(self.ctx.h, self.h, C.byref(eps), minv.ctypes.data_as(L._dp),
+                                                                 U.ctypes.data_as(L._dp), C.byref(it), rec.ctypes.data_as(L._dp),
+                                                                 C.byref(failed)))
+            return dict(eps=eps.value, Minv=np.ascontiguousarray(minv.T), cholU=np.ascontiguousarray(U.T), iteration=it.value,
+                        merged_record=rec, failed_iteration=failed.value)
         minv, rec = np.empty(self.D), np.empty(2 + 2 * self.D)
         self.ctx.check(self.ctx.lib.ahmc_pooled_state(self.ctx.h, self.h, C.byref(eps), minv.ctypes.data_as(L._dp), C.byref(it),
                                                        rec.ctypes.data_as(L._dp)))
@@ -536,13 +557,17 @@ def sample_pooled_device(rng, h: A.Hamiltonian, kappa: A.HMCKernel, theta, n_sam
     """`sample` with the pooled StanHMCAdaptor on the DEVICE: every warm-up iteration is [transition kernel, K5, all-gather,
     adaptor-update kernel] enqueued on one stream -- no device->host copy, no synchronisation, no new Hamiltonian / kernel
     objects; the sampling phase is the persistent launch.  Dynamic (NUTS) and fixed-n static trajectories (a
-    FixedIntegrationTime trajectory needs eps on the host to size the trajectory: use `sample`)."""
+    FixedIntegrationTime trajectory needs eps on the host to size the trajectory: use `sample`).
+    A DenseEuclideanMetric adapts with the pooled WelfordCov (D <= 512): M^-1 and its Cholesky factor are replaced on the
+    device at window ends; an estimate that is not positive definite raises AhmcError after the warm-up, naming the iteration."""
     import time
 
     import torch
 
-    if not isinstance(h.metric, A.DiagEuclideanMetric):
-        raise A.L.AhmcError(A.L.ERR_UNSUPPORTED, "pooled device adaptation: DiagEuclideanMetric (WelfordVar)")
+    dense = isinstance(h.metric, A.DenseEuclideanMetric)
+    if not (dense or isinstance(h.metric, A.DiagEuclideanMetric)):
+        raise A.L.AhmcError(A.L.ERR_UNSUPPORTED,
+                            "pooled device adaptation: DiagEuclideanMetric (WelfordVar) or DenseEuclideanMetric (WelfordCov)")
     tau = kappa.tau
     if isinstance(tau.termination_criterion, A.FixedIntegrationTime):
         raise A.L.AhmcError(A.L.ERR_UNSUPPORTED, "FixedIntegrationTime needs eps on the host; use sample()")
@@ -551,8 +576,8 @@ def sample_pooled_device(rng, h: A.Hamiltonian, kappa: A.HMCKernel, theta, n_sam
     tm = dict(transition=0.0, adapt=0.0, sampling_launch=0.0, bookkeeping=0.0)
     n_adapts = min(n_adapts, n_samples)
     Minv0 = h.metric.Minv if A._is_host(h.metric.Minv) else h.metric.Minv.detach().cpu().numpy()
-    ad = PooledDeviceAdaptor(dev.index or 0, D, N, n_adapts, eps0, delta, adapt_metric, *windows, Minv0=Minv0)
-    hd = A.Hamiltonian(A.DiagEuclideanMetric(ad.Minv), h.target)
+    ad = PooledDeviceAdaptor(dev.index or 0, D, N, n_adapts, eps0, delta, adapt_metric, *windows, Minv0=Minv0, dense=dense)
+    hd = A.Hamiltonian(A.DenseEuclideanMetric(ad.Minv, cholU=ad.cholU) if dense else A.DiagEuclideanMetric(ad.Minv), h.target)
     if isinstance(tau.integrator, A.JitteredLeapfrog):
         raise A.L.AhmcError(A.L.ERR_UNSUPPORTED, "JitteredLeapfrog draws its step size on the host; use sample()")
     lf_d = A.TemperedLeapfrog(ad.eps, tau.integrator.alpha) if isinstance(tau.integrator, A.TemperedLeapfrog) else A.Leapfrog(ad.eps)
@@ -575,6 +600,12 @@ def sample_pooled_device(rng, h: A.Hamiltonian, kappa: A.HMCKernel, theta, n_sam
         tm["issue_warmup"] = time.perf_counter() - t0
         torch.cuda.synchronize(dev)
     tm["transition"] = time.perf_counter() - t0  # warm-up wall time: transitions and exchanges share one stream
+    if dense and n_adapts > 0:
+        failed = ad.state()["failed_iteration"]
+        if failed:
+            ad.destroy()
+            raise A.L.AhmcError(A.L.ERR_INVALID, f"pooled WelfordCov: the adapted M^-1 of warm-up iteration {failed} is not "
+                                                 "positive definite (Cholesky failed); M^-1 and its factor kept their previous value")
     n_rest = n_samples - n_adapts
     draws = []
     if n_rest > 0:

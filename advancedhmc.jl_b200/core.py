@@ -317,26 +317,48 @@ class DiagEuclideanMetric(AbstractMetric):
 
 
 class DenseEuclideanMetric(AbstractMetric):
-    """src/metric.jl:89-120.  Minv: (D, D); cholU = cholesky(Symmetric(Minv)).U (host LAPACK via numpy)."""
+    """src/metric.jl:89-120.  Minv: (D, D); cholU = cholesky(Symmetric(Minv)).U (host LAPACK via numpy).
+    `cholU=` hands over the upper factor instead (U'U = Minv, both (D, D) as logical matrices): with CUDA tensors nothing is
+    copied to the host or factorised there and device calls read the two tensors in place (e.g. the buffers of a dense
+    `PooledDeviceAdaptor`, which change under the metric at window ends)."""
 
     kind = L.METRIC_DENSE
 
-    def __init__(self, Minv):
+    def __init__(self, Minv, cholU=None):
         if isinstance(Minv, int):
             Minv = np.eye(Minv)
+        self.Minv, self.cholU = Minv, cholU
+        if cholU is not None:
+            if tuple(Minv.shape) != tuple(cholU.shape) or Minv.ndim != 2:
+                raise L.InvalidArgument(L.ERR_INVALID, "Minv and cholU must both be D x D")
+            self.size = (Minv.shape[0],)
+            return
         Mh = Minv if _is_host(Minv) else Minv.detach().cpu().numpy()
-        self.Minv = Minv
         self._Minv_h = np.ascontiguousarray(Mh, dtype=np.float64)
         self._cholU_h = np.ascontiguousarray(np.linalg.cholesky(self._Minv_h).T)  # upper factor
         self.size = (Mh.shape[0],)
 
     def _desc(self, D, N, like):
+        if self.cholU is not None:
+            if self.size != (D,):
+                raise L.InvalidArgument(L.ERR_INVALID, f"AxesMismatch: Minv is {self.size * 2} but r has {D} rows")
+            # column-major D x D == row-major transpose; a tensor whose transpose is contiguous (the adaptor's views) is
+            # passed as it is
+            Mi, U = (_colmajor(x, like) for x in (self.Minv, self.cholU))
+            return L.Metric(L.METRIC_DENSE, _ptr(Mi), 0, _ptr(U)), (Mi, U)
         if self._Minv_h.shape != (D, D):
             raise L.InvalidArgument(L.ERR_INVALID, f"AxesMismatch: Minv is {self._Minv_h.shape} but r has {D} rows")
         # column-major D x D == transposed row-major; Minv symmetric, U stored column-major
         Mi = _coerce_like(np.ascontiguousarray(self._Minv_h.T), like)
         U = _coerce_like(np.ascontiguousarray(self._cholU_h.T), like)
         return L.Metric(L.METRIC_DENSE, _ptr(Mi), 0, _ptr(U)), (Mi, U)
+
+
+def _colmajor(a, like):
+    """the column-major buffer of the D x D matrix `a` at the residency of `like`"""
+    if not _is_host(like) and not _is_host(a) and a.device == like.device and a.dtype == torch.float64 and a.T.is_contiguous():
+        return a.T
+    return _coerce_like(a.T if _is_host(a) else a.T.contiguous(), like)
 
 
 def _coerce_like(a, like):

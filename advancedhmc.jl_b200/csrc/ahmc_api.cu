@@ -1586,10 +1586,19 @@ struct ahmc_comm {
 struct ahmc_pooled {
     int D = 0;
     int64_t N = 0;
-    char* dev = nullptr;  // one allocation: state | eps_chain | minv | w_mu | w_M2 | record | merged
+    char* dev = nullptr;  // one allocation: state | eps_chain | minv | w_mu | w_M2 | record | merged (dense: see _create_dense)
     void* state = nullptr;
     double *eps_chain = nullptr, *minv = nullptr, *w_mu = nullptr, *w_M2 = nullptr, *record = nullptr, *merged = nullptr;
     DevBuf gathered;  // R records of the last multi-rank exchange (grown on demand)
+    // dense adaptor (pooled WelfordCov): minv and cholU are D x D column-major; w_M the window's D x D accumulator, cand the
+    // candidate estimate, work the factorisation's workspace.  The host follows the schedule to launch the factorisation
+    // only at window splits.
+    bool dense = false;
+    int adapt_metric = 0;
+    int calls = 0;  // exchanges so far
+    AdaptDev sched{};
+    double *cholU = nullptr, *w_M = nullptr, *cand = nullptr, *work = nullptr;
+    size_t record_len() const { return (size_t)(2 + 2 * D) + (dense && adapt_metric ? (size_t)D * D : 0); }
 };
 
 int ahmc_comm_unique_id(ahmc_ctx* ctx, void* id128_out) {
@@ -1647,13 +1656,20 @@ int ahmc_adapt_allgather_f64(ahmc_ctx* ctx, ahmc_comm* comm, const double* recor
     return AHMC_OK;
 }
 
-int ahmc_pooled_create(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cfg* cfg, const double* Minv0, ahmc_pooled** out) {
+namespace {
+int pooled_check(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cfg* cfg, ahmc_pooled** out, AdaptDev* sched) {
     if (!ctx || !cfg || !out) return fail(ctx, AHMC_ERR_INVALID, "NULL ctx/cfg/out");
     if (D < 1 || N < 1) return fail(ctx, AHMC_ERR_INVALID, "need D >= 1, N >= 1");
     if (cfg->n_adapts < 0 || !(cfg->eps0 > 0.0)) return fail(ctx, AHMC_ERR_INVALID, "need n_adapts >= 0 and eps0 > 0");
-    AdaptDev sched{};
-    if (!stan_window_schedule(sched, cfg->init_buffer, cfg->term_buffer, cfg->window_size, cfg->n_adapts))
+    if (!stan_window_schedule(*sched, cfg->init_buffer, cfg->term_buffer, cfg->window_size, cfg->n_adapts))
         return fail(ctx, AHMC_ERR_UNSUPPORTED, "the window schedule has more than 12 window ends");
+    return AHMC_OK;
+}
+}  // namespace
+
+int ahmc_pooled_create(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cfg* cfg, const double* Minv0, ahmc_pooled** out) {
+    AdaptDev sched{};
+    if (int rc = pooled_check(ctx, D, N, cfg, out, &sched)) return rc;
     DeviceGuard g(ctx->device);
     ahmc_pooled* a = new (std::nothrow) ahmc_pooled;
     if (!a) return fail(ctx, AHMC_ERR_NOMEM, "out of host memory");
@@ -1697,8 +1713,77 @@ int ahmc_pooled_destroy(ahmc_ctx* ctx, ahmc_pooled* a) {
     delete a;
     return AHMC_OK;
 }
+int ahmc_pooled_create_dense(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cfg* cfg, const double* Minv0,
+                             ahmc_pooled** out) {
+    AdaptDev sched{};
+    if (int rc = pooled_check(ctx, D, N, cfg, out, &sched)) return rc;
+    if (D > 512) return fail(ctx, AHMC_ERR_UNSUPPORTED, "the dense pooled adaptor supports D <= 512 (got %d)", (int)D);
+    DeviceGuard g(ctx->device);
+    ahmc_pooled* a = new (std::nothrow) ahmc_pooled;
+    if (!a) return fail(ctx, AHMC_ERR_NOMEM, "out of host memory");
+    a->D = D;
+    a->N = N;
+    a->dense = true;
+    a->adapt_metric = cfg->adapt_metric ? 1 : 0;
+    a->sched = sched;
+    const size_t dd = al256((size_t)D * D * 8), rec = al256(a->record_len() * 8), rec_full = al256(((size_t)(2 + 2 * D) + (size_t)D * D) * 8);
+    const size_t total = al256(pooled_state_bytes()) + al256((size_t)N * 8) + 2 * al256((size_t)D * 8) + rec + rec_full + 5 * dd;
+    if (cudaMalloc((void**)&a->dev, total) != cudaSuccess) {
+        delete a;
+        return fail(ctx, AHMC_ERR_NOMEM, "cudaMalloc(%zu) for the pooled adaptor failed", total);
+    }
+    char* p = a->dev;
+    a->state = p; p += al256(pooled_state_bytes());
+    a->eps_chain = (double*)p; p += al256((size_t)N * 8);
+    a->w_mu = (double*)p; p += al256((size_t)D * 8);
+    a->w_M2 = (double*)p; p += al256((size_t)D * 8);
+    a->record = (double*)p; p += rec;
+    a->merged = (double*)p; p += rec_full;
+    a->minv = (double*)p; p += dd;
+    a->cholU = (double*)p; p += dd;
+    a->w_M = (double*)p; p += dd;
+    a->cand = (double*)p; p += dd;
+    a->work = (double*)p;
+    auto undo = [&](int rc) {
+        cudaStreamSynchronize(ctx->stream);
+        cudaFree(a->dev);
+        delete a;
+        return rc;
+    };
+    std::vector<char> img(pooled_state_bytes());
+    pooled_state_init(img.data(), cfg->eps0, sched, cfg->delta, cfg->gamma, cfg->t0, cfg->kappa, cfg->n_adapts, a->adapt_metric,
+                      cfg->n_min);
+    pooled_state_set_dense(img.data(), (int)a->record_len(), 0);
+    cudaError_t e = cudaMemcpyAsync(a->state, img.data(), img.size(), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->w_mu, 0, (size_t)D * 8, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->w_M2, 0, (size_t)D * 8, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->merged, 0, rec_full, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->w_M, 0, (size_t)D * D * 8, ctx->stream);
+    std::vector<double> eye;  // Minv0 == NULL: I
+    if (!Minv0) {
+        eye.assign((size_t)D * D, 0.0);
+        for (int d = 0; d < D; ++d) eye[(size_t)d * (D + 1)] = 1.0;
+    }
+    // the candidate is factorised below and, when positive definite, committed to minv / cholU
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(a->cand, Minv0 ? Minv0 : eye.data(), (size_t)D * D * 8, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = launch_fill(a->eps_chain, N, cfg->eps0, ctx->stream);
+    int nl = 0;
+    if (e == cudaSuccess) e = launch_pooled_chol(a->state, D, a->cand, a->work, a->minv, a->cholU, 1, ctx->stream, &nl);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(img.data(), a->state, img.size(), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);  // img / Minv0 / eye are host memory of this frame
+    if (e != cudaSuccess) return undo(fail(ctx, AHMC_ERR_CUDA, "creating the dense pooled adaptor: %s", cudaGetErrorString(e)));
+    ctx->launches += nl;
+    int chol_failed = 0;
+    pooled_state_read_dense(img.data(), nullptr, &chol_failed);
+    if (chol_failed) return undo(fail(ctx, AHMC_ERR_INVALID, "Minv0 is not positive definite (Cholesky pivot <= 0 or NaN)"));
+    *out = a;
+    return AHMC_OK;
+}
+
 double* ahmc_pooled_eps(ahmc_pooled* a) { return a ? a->eps_chain : nullptr; }
 double* ahmc_pooled_minv(ahmc_pooled* a) { return a ? a->minv : nullptr; }
+double* ahmc_pooled_cholu(ahmc_pooled* a) { return a && a->dense ? a->cholU : nullptr; }
 
 int ahmc_adapt_exchange_f64(ahmc_ctx* ctx, ahmc_comm* comm, ahmc_pooled* a, int32_t D, int64_t N, const double* theta,
                             int64_t ld, const double* acceptance_rate, double* eps_trace, uint32_t flags) {
@@ -1707,23 +1792,30 @@ int ahmc_adapt_exchange_f64(ahmc_ctx* ctx, ahmc_comm* comm, ahmc_pooled* a, int3
     if (D != a->D || N != a->N || ld < D) return fail(ctx, AHMC_ERR_INVALID, "D / N differ from the adaptor's, or ld < D");
     DeviceGuard g(ctx->device);
     const int R = comm ? comm->nranks : 1;
-    const size_t rec = (size_t)(2 + 2 * D);
+    const size_t rec = a->record_len();
+    const bool cov = a->dense && a->adapt_metric;  // the D x D part of the record is computed and merged
     int rc;
     if (R > 1 && (rc = grow(ctx, a->gathered, rec * 8 * (size_t)R, "gathered records"))) return rc;
-    // K5: this rank's record
+    // K5 (+ K5b for a dense adaptor): this rank's record
     int blocks;
     if ((rc = adapt_workspace(ctx, D, N, &blocks))) return rc;
     double* ws = (double*)ctx->adapt_scratch.p;
     int nl = 0;
     CU(launch_adapt_summary(D, N, theta, ld, acceptance_rate, a->record, ws + 2, (unsigned*)ws, blocks, ctx->stream, &nl));
+    if (cov) CU(launch_adapt_cov(D, N, theta, ld, a->record + 2, a->record + 2 + 2 * D, ctx->stream, &nl));
     const double* gathered = a->record;
     if (R > 1) {
         if ((rc = nccl_allgather_f64(a->record, (double*)a->gathered.p, rec, comm->nccl, ctx->stream)))
             return fail(ctx, AHMC_ERR_CUDA, "ncclAllGather: %s", nccl_err(rc));
         gathered = (double*)a->gathered.p;
     }
-    CU(launch_pooled_update(a->state, gathered, R, D, a->w_mu, a->w_M2, a->minv, a->eps_chain, N, eps_trace, a->merged,
-                            ctx->stream, &nl));
+    // dense: the D x D merge / push reads the window's n and mean before pooled_update_kernel advances them
+    if (cov) CU(launch_pooled_cov(a->state, gathered, R, D, a->w_mu, a->w_M, a->cand, a->merged, ctx->stream, &nl));
+    CU(launch_pooled_update(a->state, gathered, R, D, a->w_mu, a->w_M2, a->dense ? nullptr : a->minv, a->eps_chain, N, eps_trace,
+                            a->merged, ctx->stream, &nl));
+    a->calls += 1;
+    if (cov && pooled_chol_due(a->sched, a->adapt_metric, a->calls))
+        CU(launch_pooled_chol(a->state, D, a->cand, a->work, a->minv, a->cholU, 0, ctx->stream, &nl));
     ctx->launches += nl;
     if (!(flags & AHMC_FLAG_ASYNC)) CU(cudaStreamSynchronize(ctx->stream));
     return AHMC_OK;
@@ -1731,6 +1823,7 @@ int ahmc_adapt_exchange_f64(ahmc_ctx* ctx, ahmc_comm* comm, ahmc_pooled* a, int3
 
 int ahmc_pooled_state(ahmc_ctx* ctx, ahmc_pooled* a, double* eps, double* Minv, int32_t* iteration, double* merged_record) {
     if (!ctx || !a) return fail(ctx, AHMC_ERR_INVALID, "NULL ctx/adaptor");
+    if (a->dense) return fail(ctx, AHMC_ERR_INVALID, "dense pooled adaptor: read it with ahmc_pooled_state_dense");
     DeviceGuard g(ctx->device);
     std::vector<char> img(pooled_state_bytes());
     CU(cudaMemcpyAsync(img.data(), a->state, img.size(), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1740,6 +1833,27 @@ int ahmc_pooled_state(ahmc_ctx* ctx, ahmc_pooled* a, double* eps, double* Minv, 
     int it = 0;
     pooled_state_read(img.data(), eps, &it, nullptr, nullptr);
     if (iteration) *iteration = it;
+    return AHMC_OK;
+}
+
+int ahmc_pooled_state_dense(ahmc_ctx* ctx, ahmc_pooled* a, double* eps, double* Minv, double* cholU, int32_t* iteration,
+                            double* merged_record, int32_t* failed_iteration) {
+    if (!ctx || !a) return fail(ctx, AHMC_ERR_INVALID, "NULL ctx/adaptor");
+    if (!a->dense) return fail(ctx, AHMC_ERR_INVALID, "diagonal pooled adaptor: read it with ahmc_pooled_state");
+    DeviceGuard g(ctx->device);
+    const size_t dd = (size_t)a->D * a->D * 8;
+    std::vector<char> img(pooled_state_bytes());
+    CU(cudaMemcpyAsync(img.data(), a->state, img.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    if (Minv) CU(cudaMemcpyAsync(Minv, a->minv, dd, cudaMemcpyDeviceToHost, ctx->stream));
+    if (cholU) CU(cudaMemcpyAsync(cholU, a->cholU, dd, cudaMemcpyDeviceToHost, ctx->stream));
+    if (merged_record)
+        CU(cudaMemcpyAsync(merged_record, a->merged, (size_t)(2 + 2 * a->D) * 8 + dd, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    int it = 0, failed = 0;
+    pooled_state_read(img.data(), eps, &it, nullptr, nullptr);
+    pooled_state_read_dense(img.data(), &failed, nullptr);
+    if (iteration) *iteration = it;
+    if (failed_iteration) *failed_iteration = failed;
     return AHMC_OK;
 }
 

@@ -293,8 +293,15 @@ struct NcclId {
 cudaError_t launch_pooled_update(void* state, const double* gathered, int R, int D, double* w_mu, double* w_M2, double* Minv,
                                  double* eps_chain, long long N, double* eps_trace, double* merged_out, cudaStream_t st,
                                  int* n_launches);
+cudaError_t launch_pooled_cov(void* state, const double* gathered, int R, int D, const double* w_mu, double* w_M, double* cand,
+                              double* merged_out, cudaStream_t st, int* n_launches);
+cudaError_t launch_pooled_chol(void* state, int D, const double* cand, double* work, double* Minv, double* cholU, int force,
+                               cudaStream_t st, int* n_launches);
 cudaError_t launch_fill(double* p, long long n, double v, cudaStream_t st);
 size_t pooled_state_bytes();
+void pooled_state_set_dense(void* host_image, int record_len, int cand_ready);
+void pooled_state_read_dense(const void* host_image, int* failed_iteration, int* chol_failed);
+bool pooled_chol_due(const AdaptDev& sched, int adapt_metric, int i);
 void pooled_state_init(void* host_image, double eps0, const AdaptDev& sched, double delta, double gamma, double t0, double kappa,
                        int n_adapts, int adapt_metric, int n_min);
 void pooled_state_read(const void* host_image, double* eps, int* iteration, int* m, double* n_window);

@@ -9,6 +9,15 @@
 //                             (massmatrix.jl:141-157, n_min :60-62), the Stan window schedule
 //                             (stan_adaptor.jl:13-50, 137-159); eps and M^-1 are written straight into the device buffers
 //                             the next transition reads (eps_chain[N], Minv[D]).
+// A dense adaptor (pooled `WelfordCov`, massmatrix.jl:286-340) records (2 + 2D + D^2) doubles per rank (K5 + K5b), and
+// runs, in this order:
+//     pooled_cov_kernel       rank-ordered merge of the D x D blocks, push into the window's D x D accumulator and, at an
+//                             update, the regularised estimate into a scratch candidate -- BEFORE pooled_update_kernel,
+//                             which advances i, n and the window mean it reads
+//     pooled_update_kernel    as above, with Minv == nullptr (the diagonal estimate is not written)
+//     pooled_chol_kernel      only at window splits inside the metric window: factorises the candidate and, if every
+//                             pivot is > 0, commits M^-1 and its upper factor U together; otherwise keeps both and
+//                             records the iteration (`cholesky` throws PosDefException there, metric.jl:104-108).
 // NCCL is bound at run time (dlopen): the library loads without it and a Julia host can hand over the communicator it
 // already owns (NCCL.jl) or let ahmc_comm_create make one from a broadcast unique id.
 #ifndef AHMC_SIMT_EMULATION
@@ -36,15 +45,36 @@ struct PooledState {
     int splits[16];
     int adapt_metric, n_min;
     int finalized;
+    // dense adaptor only (zero = diagonal adaptor)
+    int record_len;        // doubles per rank in `gathered`; 0 = 2 + 2D
+    int cand_ready;        // pooled_cov_kernel wrote a new estimate to the candidate; pooled_chol_kernel consumes it
+    int chol_failed;       // the last factorisation found a pivot <= 0 or NaN
+    int failed_iteration;  // first iteration whose factorisation failed (0 = never)
 };
 
-// one CTA.  gathered: R records of (2 + 2D) doubles in rank order.
+// schedule of iteration st->i + 1 (stan_adaptor.jl:137-159), shared by every kernel of one exchange
+struct PooledStep {
+    bool push, update, reset;
+};
+__device__ inline PooledStep pooled_schedule(const PooledState* st) {
+    const int i = st->i + 1;
+    bool split = false;
+    for (int k = 0; k < st->n_splits; ++k) split |= (st->splits[k] == i);
+    PooledStep s;
+    s.push = st->adapt_metric && i >= st->window_start && i <= st->window_end;
+    s.update = s.push && split;
+    s.reset = split;
+    return s;
+}
+
+// one CTA.  gathered: R records of st->record_len (default 2 + 2D) doubles in rank order.  Minv == nullptr: the estimate is
+// not written (dense adaptor: pooled_cov_kernel owns M^-1).
 __global__ void __launch_bounds__(256) pooled_update_kernel(PooledState* st, const double* __restrict__ gathered, int R, int D,
                                                             double* w_mu, double* w_M2, double* Minv, double* eps_chain,
                                                             long long N, double* eps_trace, double* merged_out) {
     __shared__ double s_n, s_alpha;
     __shared__ int s_push, s_update, s_reset;
-    const int rec = 2 + 2 * D;
+    const int rec = st->record_len ? st->record_len : 2 + 2 * D;
     // ---- rank-ordered Chan merge of the R records (adaptation.py merge_records; fixed order => identical on all ranks)
     if (threadIdx.x == 0) {
         double n = gathered[0], a = gathered[1];
@@ -61,12 +91,10 @@ __global__ void __launch_bounds__(256) pooled_update_kernel(PooledState* st, con
     }
     // schedule decisions of THIS iteration (stan_adaptor.jl:137-159)
     if (threadIdx.x == 0) {
-        const int i = st->i + 1;
-        bool split = false;
-        for (int k = 0; k < st->n_splits; ++k) split |= (st->splits[k] == i);
-        s_push = st->adapt_metric && i >= st->window_start && i <= st->window_end;
-        s_update = s_push && split;
-        s_reset = split;
+        const PooledStep s = pooled_schedule(st);
+        s_push = s.push;
+        s_update = s.update;
+        s_reset = s.reset;
     }
     __syncthreads();
     const bool push = s_push != 0, update = s_update != 0, reset = s_reset != 0;
@@ -89,7 +117,7 @@ __global__ void __launch_bounds__(256) pooled_update_kernel(PooledState* st, con
             const double dl = mean - w_mu[d];
             double M = w_M2[d] + M2 + dl * dl * (na * nb / n);
             double mu = w_mu[d] + dl * (nb / n);
-            if (update && n >= (double)st->n_min)  // get_estimation (massmatrix.jl:152-157)
+            if (Minv && update && n >= (double)st->n_min)  // get_estimation (massmatrix.jl:152-157)
                 Minv[d] = n / ((n + 5.0) * (n - 1.0)) * M + 1e-3 * (5.0 / (n + 5.0));
             if (reset) {
                 M = 0.0;
@@ -142,6 +170,111 @@ __global__ void __launch_bounds__(256) pooled_update_kernel(PooledState* st, con
     for (long long c = threadIdx.x; c < N; c += blockDim.x) eps_chain[c] = e;
 }
 
+// Dense adaptor, step 1 of the exchange (before pooled_update_kernel).  Any grid; one thread per entry e = i + D*j of the
+// column-major D x D blocks (coalesced).  gathered: R records [n, sum alpha, mean[D], M2diag[D], M2full[D*D]].
+//   * rank-ordered Chan merge of the D x D blocks, the same arithmetic and order as adaptation.merge_records(.., "cov"): each
+//     rank's step uses the running means BEFORE that rank is merged;
+//   * WelfordCov push_record into w_M with the window's n and mean BEFORE this iteration (st->n, w_mu);
+//   * at an update with n >= n_min, get_estimation (massmatrix.jl:335-340) into `cand`, and st->cand_ready = 1;
+//   * at a split, w_M restarts from zero.
+__global__ void __launch_bounds__(256) pooled_cov_kernel(PooledState* st, const double* __restrict__ gathered, int R, int D,
+                                                         const double* __restrict__ w_mu, double* w_M, double* cand,
+                                                         double* merged_out) {
+    const int rec = st->record_len;
+    const PooledStep s = pooled_schedule(st);
+    double n_b = gathered[0];
+    for (int r = 1; r < R; ++r) n_b += gathered[(size_t)r * rec];
+    const double n_w = st->n, n = n_w + n_b;
+    const bool update = s.update && n >= (double)st->n_min;
+    if (blockIdx.x == 0 && threadIdx.x == 0) st->cand_ready = update;
+    const long long DD = (long long)D * D;
+    const double c = n / ((n + 5.0) * (n - 1.0)), reg = 1e-3 * (5.0 / (n + 5.0)), wt = n_w * n_b / n;
+    for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < DD; e += (long long)gridDim.x * blockDim.x) {
+        const int i = (int)(e % D), j = (int)(e / D);
+        const size_t off = 2 + 2 * (size_t)D + (size_t)e;
+        double n_a = gathered[0], mi = gathered[2 + i], mj = gathered[2 + j], M = gathered[off];
+        for (int r = 1; r < R; ++r) {
+            const double* g = gathered + (size_t)r * rec;
+            const double nb = g[0], nn = n_a + nb, w = n_a * nb / nn;
+            const double di = g[2 + i] - mi, dj = g[2 + j] - mj;
+            M += g[off] + di * dj * w;
+            mi += di * (nb / nn);
+            mj += dj * (nb / nn);
+            n_a = nn;
+        }
+        if (merged_out) merged_out[off] = M;
+        if (s.push) {
+            const double di = mi - w_mu[i], dj = mj - w_mu[j];
+            const double W = w_M[e] + M + di * dj * wt;
+            if (update) cand[e] = c * W + (i == j ? reg : 0.0);
+            w_M[e] = s.reset ? 0.0 : W;
+        } else if (s.reset) {
+            w_M[e] = 0.0;
+        }
+    }
+}
+
+// Dense adaptor, step 3 (window splits inside the metric window only; once at creation with force = 1).  One CTA, D <= 512.
+// Consumes st->cand_ready.  Factorises cand = U^T U reading only its upper triangle (cholesky(Symmetric(M^-1)).U,
+// metric.jl:104-108, 117) by the column Cholesky-Crout recurrence on L = U^T, kept column-major in `work` so that the
+// threads (one per row) read it coalesced; every sum has a fixed order.  The pivot test is LAPACK potrf's: a pivot <= 0 or
+// NaN fails.  On success cand -> Minv and U -> cholU (column-major, zero below the diagonal), both at once; on failure
+// both keep their previous values and the first failing iteration is recorded.
+constexpr int kCholThreads = 512;
+__global__ void __launch_bounds__(kCholThreads) pooled_chol_kernel(PooledState* st, int D, const double* __restrict__ cand,
+                                                                   double* work, double* Minv, double* cholU, int force) {
+    __shared__ int s_go;
+    __shared__ double s_piv;
+    if (threadIdx.x == 0) {
+        s_go = force || st->cand_ready;
+        st->cand_ready = 0;
+    }
+    __syncthreads();
+    if (!s_go) return;
+    bool ok = true;
+    for (int j = 0; j < D; ++j) {
+        const double* Lj = work + j;  // row j of L: Lj[D * k]
+        for (int i = threadIdx.x; i < D; i += blockDim.x) {
+            if (i < j) continue;
+            const double* Li = work + i;
+            double d0 = 0.0, d1 = 0.0;
+            int k = 0;
+            for (; k + 1 < j; k += 2) {
+                d0 = fma(Li[(size_t)D * k], Lj[(size_t)D * k], d0);
+                d1 = fma(Li[(size_t)D * (k + 1)], Lj[(size_t)D * (k + 1)], d1);
+            }
+            if (k < j) d0 = fma(Li[(size_t)D * k], Lj[(size_t)D * k], d0);
+            const double v = cand[j + (size_t)D * i] - (d0 + d1);  // A[j][i], j <= i: upper triangle
+            if (i == j) s_piv = v;
+            else work[i + (size_t)D * j] = v;
+        }
+        __syncthreads();
+        const double piv = s_piv;
+        if (!(piv > 0.0)) {  // the same value in every thread: the whole block leaves together
+            ok = false;
+            break;
+        }
+        const double ljj = sqrt(piv);
+        for (int i = threadIdx.x; i < D; i += blockDim.x) {
+            if (i < j) continue;
+            work[i + (size_t)D * j] = i == j ? ljj : work[i + (size_t)D * j] / ljj;
+        }
+        __syncthreads();
+    }
+    if (ok) {
+        const long long DD = (long long)D * D;
+        for (long long e = threadIdx.x; e < DD; e += blockDim.x) {
+            const int r = (int)(e % D), c = (int)(e / D);
+            Minv[e] = cand[e];
+            cholU[e] = r <= c ? work[c + (size_t)D * r] : 0.0;
+        }
+    }
+    if (threadIdx.x == 0) {
+        st->chol_failed = !ok;
+        if (!ok && !force && st->failed_iteration == 0) st->failed_iteration = st->i;
+    }
+}
+
 #ifndef AHMC_SIMT_EMULATION  // host launch code and the NCCL binding (skipped by the CPU SIMT emulation harness, tests/simt_emu/)
 __global__ void fill_kernel(double* p, long long n, double v) {
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) p[i] = v;
@@ -151,6 +284,21 @@ cudaError_t launch_pooled_update(void* state, const double* gathered, int R, int
                                  double* eps_chain, long long N, double* eps_trace, double* merged_out, cudaStream_t st,
                                  int* n_launches) {
     pooled_update_kernel<<<1, 256, 0, st>>>((PooledState*)state, gathered, R, D, w_mu, w_M2, Minv, eps_chain, N, eps_trace, merged_out);
+    if (n_launches) *n_launches += 1;
+    return cudaGetLastError();
+}
+cudaError_t launch_pooled_cov(void* state, const double* gathered, int R, int D, const double* w_mu, double* w_M, double* cand,
+                              double* merged_out, cudaStream_t st, int* n_launches) {
+    const long long DD = (long long)D * D;
+    const unsigned blocks = (unsigned)((DD + 255) / 256 < 4096 ? (DD + 255) / 256 : 4096);
+    pooled_cov_kernel<<<blocks, 256, 0, st>>>((PooledState*)state, gathered, R, D, w_mu, w_M, cand, merged_out);
+    if (n_launches) *n_launches += 1;
+    return cudaGetLastError();
+}
+cudaError_t launch_pooled_chol(void* state, int D, const double* cand, double* work, double* Minv, double* cholU, int force,
+                               cudaStream_t st, int* n_launches) {
+    const int threads = D >= kCholThreads ? kCholThreads : (D + 31) / 32 * 32;
+    pooled_chol_kernel<<<1, threads, 0, st>>>((PooledState*)state, D, cand, work, Minv, cholU, force);
     if (n_launches) *n_launches += 1;
     return cudaGetLastError();
 }
@@ -182,6 +330,26 @@ void pooled_state_init(void* host_image, double eps0, const AdaptDev& sched, dou
     s.n_min = n_min;
     s.finalized = 0;
     memcpy(host_image, &s, sizeof s);
+}
+void pooled_state_set_dense(void* host_image, int record_len, int cand_ready) {
+    PooledState s;
+    memcpy(&s, host_image, sizeof s);
+    s.record_len = record_len;
+    s.cand_ready = cand_ready;
+    memcpy(host_image, &s, sizeof s);
+}
+void pooled_state_read_dense(const void* host_image, int* failed_iteration, int* chol_failed) {
+    PooledState s;
+    memcpy(&s, host_image, sizeof s);
+    if (failed_iteration) *failed_iteration = s.failed_iteration;
+    if (chol_failed) *chol_failed = s.chol_failed;
+}
+// host-side schedule of the dense adaptor's factorisation: iteration i is a window split inside the metric window
+bool pooled_chol_due(const AdaptDev& sched, int adapt_metric, int i) {
+    if (!adapt_metric || i < sched.window_start || i > sched.window_end) return false;
+    for (int k = 0; k < sched.n_splits; ++k)
+        if (sched.splits[k] == i) return true;
+    return false;
 }
 void pooled_state_read(const void* host_image, double* eps, int* iteration, int* m, double* n_window) {
     PooledState s;

@@ -330,8 +330,29 @@ double* ahmc_pooled_minv(ahmc_pooled* a);
 int ahmc_adapt_exchange_f64(ahmc_ctx* ctx, ahmc_comm* comm, ahmc_pooled* a, int32_t D, int64_t N, const double* theta,
                             int64_t ld, const double* acceptance_rate, double* eps_trace, uint32_t flags);
 /* synchronising read-back of the adaptor (host outputs, each nullable): current eps, Minv[D], iterations done,
- * the merged record [n, sum alpha, mean[D], M2[D]] of the last exchange */
+ * the merged record [n, sum alpha, mean[D], M2[D]] of the last exchange.  A dense adaptor -> AHMC_ERR_INVALID
+ * (use ahmc_pooled_state_dense). */
 int ahmc_pooled_state(ahmc_ctx* ctx, ahmc_pooled* a, double* eps, double* Minv, int32_t* iteration, double* merged_record);
+
+/* StanHMCAdaptor(WelfordCov, NesterovDualAveraging) pooled over all chains of all ranks, on the device (massmatrix.jl:286-340).
+ * Minv0: host, D x D column-major, symmetric positive definite; NULL = I.  1 <= D <= 512 (the dense operators' bound):
+ * D > 512 -> AHMC_ERR_UNSUPPORTED; a Minv0 whose Cholesky factorisation fails -> AHMC_ERR_INVALID (creation synchronises).
+ *   ahmc_pooled_minv(a)  : Minv[D x D] column-major     -> ahmc_metric{AHMC_METRIC_DENSE, Minv, 0, cholU}
+ *   ahmc_pooled_cholu(a) : cholU[D x D] column-major upper factor, U'U = Minv (NULL for a diagonal adaptor)
+ * ahmc_adapt_exchange_f64 records [n, sum alpha, mean[D], M2diag[D], M2full[D*D]] (K5 + K5b, adapt_metric = 1) or the
+ * diagonal record (adapt_metric = 0: step size only, Minv0 and its factor are never touched).  Minv changes only at a window
+ * split inside the metric window with n >= n_min, to n/((n+5)(n-1)) M + 1e-3 (5/(n+5)) I, and cholU with it: the new
+ * estimate is factorised on the device (upper triangle only) and committed with its factor only if every pivot is > 0;
+ * otherwise both keep their previous values and the iteration is recorded as `failed_iteration` (first failure only). */
+int ahmc_pooled_create_dense(ahmc_ctx* ctx, int32_t D, int64_t N, const ahmc_pooled_cfg* cfg, const double* Minv0,
+                             ahmc_pooled** out);
+double* ahmc_pooled_cholu(ahmc_pooled* a);
+/* synchronising read-back of a dense adaptor (host outputs, each nullable): eps, Minv[D*D], cholU[D*D] (column-major),
+ * iterations done, the merged record [n, sum alpha, mean[D], M2diag[D], M2full[D*D]] of the last exchange (the D x D part
+ * stays zero with adapt_metric = 0), the first iteration whose factorisation failed (0 = never).  A diagonal adaptor ->
+ * AHMC_ERR_INVALID. */
+int ahmc_pooled_state_dense(ahmc_ctx* ctx, ahmc_pooled* a, double* eps, double* Minv, double* cholU, int32_t* iteration,
+                            double* merged_record, int32_t* failed_iteration);
 
 /* ---- adaptor statistics (src/adaptation) ------------------------------------------------------ */
 /* Pooled summary of one iteration over this GPU's N chains, written to a small device/host record that

@@ -598,4 +598,57 @@ function destroy!(a::B200PooledAdaptor)
     return nothing
 end
 
+"""
+Pooled `StanHMCAdaptor(WelfordCov, NesterovDualAveraging)` resident on the device (massmatrix.jl:286-340): the dense form of
+`B200PooledAdaptor`.  `M⁻¹` and `U` (upper, `U'U = M⁻¹`) are D x D CuArray views of the buffers the library updates in place
+at window ends (the new estimate is factorised on the device; a failed factorisation keeps both and is reported by
+`b200_pooled_state(::B200PooledDenseAdaptor)` as `failed_iteration`).  Build the metric once from them, e.g.
+`DenseEuclideanMetric(a.M⁻¹)` with the transition calls passing `CMetric(METRIC_DENSE, dptr(a.M⁻¹), 0, dptr(a.U))`.
+Like the rest of this file, written but not executed.
+"""
+mutable struct B200PooledDenseAdaptor
+    h::Ptr{Cvoid}
+    D::Int
+    N::Int
+    ϵ::CuVector{Float64}
+    M⁻¹::CuMatrix{Float64}
+    U::CuMatrix{Float64}
+end
+function b200_pooled_adaptor(D::Integer, N::Integer, n_adapts::Integer, ϵ0::Real, M⁻¹0::Union{Nothing,Matrix{Float64}};
+                             δ=0.8, adapt_metric=true, init_buffer=75, term_buffer=50, window_size=25, γ=0.05, t_0=10.0,
+                             κ=0.75, n_min=10)
+    cfg = Ref(CPooledCfg(n_adapts, init_buffer, term_buffer, window_size, δ, γ, t_0, κ, ϵ0, adapt_metric ? 1 : 0, n_min))
+    out = Ref{Ptr{Cvoid}}(C_NULL)
+    GC.@preserve M⁻¹0 check(ccall((:ahmc_pooled_create_dense, libahmc), Cint,
+                                  (Ptr{Cvoid}, Int32, Int64, Ref{CPooledCfg}, Ptr{Float64}, Ref{Ptr{Cvoid}}),
+                                  context().h, D, N, cfg, M⁻¹0 === nothing ? C_NULL : pointer(M⁻¹0), out))
+    pe = ccall((:ahmc_pooled_eps, libahmc), Ptr{Float64}, (Ptr{Cvoid},), out[])
+    pm = ccall((:ahmc_pooled_minv, libahmc), Ptr{Float64}, (Ptr{Cvoid},), out[])
+    pu = ccall((:ahmc_pooled_cholu, libahmc), Ptr{Float64}, (Ptr{Cvoid},), out[])
+    ϵ = unsafe_wrap(CuArray, reinterpret(CuPtr{Float64}, pe), (Int(N),))
+    Mi = unsafe_wrap(CuArray, reinterpret(CuPtr{Float64}, pm), (Int(D), Int(D)))  # column-major, as Julia's
+    U = unsafe_wrap(CuArray, reinterpret(CuPtr{Float64}, pu), (Int(D), Int(D)))
+    return B200PooledDenseAdaptor(out[], D, N, ϵ, Mi, U)
+end
+function AdvancedHMC.Adaptation.adapt!(a::B200PooledDenseAdaptor, c::Union{Nothing,B200Comm}, θ::CuMatrix{Float64}, α::CuVector{Float64})
+    GC.@preserve θ α check(ccall((:ahmc_adapt_exchange_f64, libahmc), Cint,
+                                 (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int32, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, UInt32),
+                                 context().h, c === nothing ? C_NULL : c.h, a.h, a.D, a.N, dptr(θ), a.D, dptr(α), C_NULL, FLAG_ASYNC))
+    return nothing
+end
+"synchronising read-back: (ϵ, M⁻¹, U, iterations done, failed_iteration); failed_iteration = 0 when every factorisation succeeded"
+function b200_pooled_state(a::B200PooledDenseAdaptor)
+    ϵ = Ref{Float64}(0.0); it = Ref{Int32}(0); failed = Ref{Int32}(0)
+    Mi = zeros(Float64, a.D, a.D); U = zeros(Float64, a.D, a.D)
+    GC.@preserve Mi U check(ccall((:ahmc_pooled_state_dense, libahmc), Cint,
+                                  (Ptr{Cvoid}, Ptr{Cvoid}, Ref{Float64}, Ptr{Float64}, Ptr{Float64}, Ref{Int32}, Ptr{Float64}, Ref{Int32}),
+                                  context().h, a.h, ϵ, pointer(Mi), pointer(U), it, C_NULL, failed))
+    return ϵ[], Mi, U, Int(it[]), Int(failed[])
+end
+function destroy!(a::B200PooledDenseAdaptor)
+    check(ccall((:ahmc_pooled_destroy, libahmc), Cint, (Ptr{Cvoid}, Ptr{Cvoid}), context().h, a.h))
+    a.h = C_NULL
+    return nothing
+end
+
 end # module
